@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps 5 ...     # the reference's CPU path (C restatement, host cores)
     torchrun --nproc-per-node N bench.py --gpus N ...           # N GPUs: weak series (1e8 rows per GPU) + strong series
     python bench.py --config 3|4|5 [--gpus N]                   # the other BASELINE configs (benchmarks/configs_bench.py)
+    python bench.py ... --dump-outputs DIR                      # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input:
     c = ScalarFunctions::add(a, b)   (25 chunks x 4e6 rows of Float64, no nulls)   -> 24 B/row through HBM
@@ -160,6 +161,27 @@ def env_ranks():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
 
 
+DUMP_ROWS = 1 << 22   # rows of c that --dump-outputs writes: 32 MB of float64
+
+
+def dump_rows(n: int) -> np.ndarray:
+    """The row numbers of c that --dump-outputs writes, for a c of n rows: drawn with a fixed seed, the same on every run."""
+    return np.sort(np.random.default_rng(SEED).integers(0, n, min(DUMP_ROWS, n)))
+
+
+def dump_outputs(out_dir: str, c_chunks, s: float, count: int):
+    """--dump-outputs: what the last timed step returned to its caller, so that two builds can be compared output for output.
+    c.npy holds the values of c at the rows dump_rows picks (c has no nulls in this workload, so it carries no validity),
+    sum.npy holds sum(c) and count.npy the number of rows it counted.  At N > 1 rank 0 writes what its caller receives:
+    its own shard of c beside the sum and count combined over every rank."""
+    c = np.concatenate(c_chunks)
+    rows = dump_rows(c.shape[0])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "c.npy"), c[rows])
+    np.save(os.path.join(out_dir, "sum.npy"), np.array([s], np.float64))
+    np.save(os.path.join(out_dir, "count.npy"), np.array([count], np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------
 # CPU arm: the reference's CPU path (C restatement in oracle/, see oracle/oracle.h for provenance)
 
@@ -212,8 +234,11 @@ def run_reference_arm(args, rank: int, world: int):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        s = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs is not None:
+        _, _, bufs, _, _, outs, _ = step._keep
+        dump_outputs(args.dump_outputs, [v for v, _ in bufs], s, sum(len(v) - outs[i].null_count for i, (v, _) in enumerate(bufs)))
     value = rows * args.steps / dt
     sample = (f"{rows} rows ({rows // CHUNK} chunks x {CHUNK}) per step, {args.steps} steps; add on {threads} threads (one per chunk, rayon mirror), "
               f"sum on 1 thread; output buffers allocated once")
@@ -261,11 +286,15 @@ class HotLoop:
         self.N, self.a, self.b, self.depth = N, a, b, depth
         self.inflight = []
         self.last = None
+        self.last_c = None
 
-    def retire(self):
+    def retire(self, keep: bool = False):
         c, fut = self.inflight.pop(0)
         r = fut.result()
-        c.free()
+        if keep:
+            self.last_c = c
+        else:
+            c.free()
         self.last = (float(r["sum"]), int(r["count"]), int(r["rows"]))
 
     def step(self):
@@ -273,19 +302,20 @@ class HotLoop:
         if len(self.inflight) > self.depth:
             self.retire()
 
-    def drain(self):
+    def drain(self, keep_last: bool = False):
+        """keep_last: the last step's c is left allocated in last_c (for --dump-outputs) instead of freed."""
         while self.inflight:
-            self.retire()
+            self.retire(keep=keep_last and len(self.inflight) == 1)
         return self.last
 
 
-def timed_loop(ctx, loop: HotLoop, steps: int, world: int):
+def timed_loop(ctx, loop: HotLoop, steps: int, world: int, keep_last: bool = False):
     """barrier; K steps between two events on the compute stream; drain; barrier.  Returns max-over-ranks ms."""
     ctx.comm_barrier()
     ctx.timer_start()
     for _ in range(steps):
         loop.step()
-    loop.drain()
+    loop.drain(keep_last)
     ms = ctx.timer_stop()
     ctx.comm_barrier()
     if world > 1:
@@ -371,7 +401,7 @@ def run_gpu_arm(args, rank: int, world: int, local: int):
     launches0 = ctx.launch_count()
     coll0 = ctx.comm_info()["collectives"]
     t_wall0 = time.perf_counter()
-    ms = timed_loop(ctx, loop, args.steps, world)
+    ms = timed_loop(ctx, loop, args.steps, world, keep_last=args.dump_outputs is not None)
     t_wall1 = time.perf_counter()
     launches = ctx.launch_count() - launches0
     collectives = ctx.comm_info()["collectives"] - coll0
@@ -391,6 +421,11 @@ def run_gpu_arm(args, rank: int, world: int, local: int):
     sampler.join(timeout=1)
     clocks = sampler.summary(t_wall0, t_wall2)
     clocks["window"] = f"timed region + {extra} untimed steps of the same load"
+    if loop.last_c is not None:
+        if rank == 0:   # at N > 1, c is rank 0's shard and the sum is the combined one
+            dump_outputs(args.dump_outputs, [x.value_slice() for x in loop.last_c.download()], last[0], last[1])
+        loop.last_c.free()
+        loop.last_c = None
 
     # ---- the same series with the other transport of the combine (N > 1) ----
     other_transport = None
@@ -574,10 +609,17 @@ def run_cpu_baseline():
         return {"value": None, "unit": "rows/s", "cores": 0, "kind": "port", "sample": f"failed: {e}"}
 
 
+def _positive_int(s: str) -> int:
+    n = int(s)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=_positive_int, default=100, help="timed steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scaling", default=None, choices=["weak", "strong"],
@@ -586,7 +628,11 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only: skip the host-buffer leg")
     ap.add_argument("--skip-cpu", action="store_true", help="profiling runs only: skip the CPU baseline leg")
     ap.add_argument("--skip-other-series", action="store_true", help="N > 1: measure only the primary scaling series")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/{c,sum,count}.npy (c: a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.dump_outputs is not None and args.config != 1:
+        ap.error("--dump-outputs applies to the headline workload (--config 1)")
     if args.scaling is None:
         args.scaling = "weak" if args.config == 1 else "strong"
     rank, world, local = env_ranks()

@@ -211,9 +211,7 @@ def config5_run(rdf, N, parallel, ctx, rank, world, args):
             c.free()
         return a, b
 
-    steps = max(1, min(args.steps, 5))
-    args.steps = steps
-    ms, last, launches, recs = _time(ctx, step, steps, min(args.warmup, 2), world, N)
+    ms, last, launches, recs = _time(ctx, step, args.steps, min(args.warmup, 2), world, N)
     a, b = last
     check = {"i2_sum": int(a["sum"]), "i2_min": int(a["min"]), "i2_max": int(a["max"]), "i2_count": int(a["count"]), "f7_sum": float(b["sum"]),
              "f7_count": int(b["count"]), "rows": int(b["rows"])}
@@ -222,45 +220,52 @@ def config5_run(rdf, N, parallel, ctx, rank, world, args):
 
 
 def reference_arm(args, rank):
-    """The reference's CPU path for the config (oracle port), bounded sample: ONE chunk of 4e6 rows per column, scaled."""
+    """The reference's CPU path for the config (oracle port), bounded sample: ONE chunk of 4e6 rows per column, scaled.
+    A step is one pass of the config's operators over that chunk; --warmup untimed passes, then --steps timed ones."""
     if rank != 0:
         return
     from oracle import pyoracle as orc
 
     cfg = args.config
-    t0 = time.perf_counter()
     if cfg == 3:
         cols = [[orc.generate(orc.I64, 2 if k == 7 else 3, 0, 0, SEED, 30 + k, 0, CHUNK, 10)] for k in range(8)]
-        t0 = time.perf_counter()
-        for c in cols:   # sum, max, min are separate sequential passes; count is metadata (aggregate.rs:12-31,70-93)
-            for op in (orc.SUM, orc.MAX, orc.MIN, orc.COUNT):
-                orc.aggregate(op, orc.I64, c)
-        threads = 1
+
+        def step():
+            for c in cols:   # sum, max, min are separate sequential passes; count is metadata (aggregate.rs:12-31,70-93)
+                for op in (orc.SUM, orc.MAX, orc.MIN, orc.COUNT):
+                    orc.aggregate(op, orc.I64, c)
     elif cfg == 4:
         x = [orc.generate(orc.I32, 2, 0, 0, SEED, 40, 0, CHUNK, 10)]
         y = [orc.generate(orc.F64, 0, -1e3, 1e3, SEED, 41, 0, CHUNK)]
-        t0 = time.perf_counter()
-        _, xf = orc.col_cast(orc.I32, orc.F64, x)
-        _, z = orc.col_binary(orc.ADD, orc.F64, xf, y)
-        _, w = orc.col_binary(orc.MUL, orc.F64, z, y)
-        orc.aggregate(orc.SUM, orc.F64, w)
-        threads = 1
+
+        def step():
+            _, xf = orc.col_cast(orc.I32, orc.F64, x)
+            _, z = orc.col_binary(orc.ADD, orc.F64, xf, y)
+            _, w = orc.col_binary(orc.MUL, orc.F64, z, y)
+            orc.aggregate(orc.SUM, orc.F64, w)
     else:
         i0 = [orc.generate(orc.I64, 3, 0, 0, SEED, 50, 0, CHUNK, 20)]; i1 = [orc.generate(orc.I64, 3, 0, 0, SEED, 51, 0, CHUNK, 20)]
         f0 = [orc.generate(orc.F64, 0, -1e3, 1e3, SEED, 52, 0, CHUNK, 20)]; f1 = [orc.generate(orc.F64, 1, 0, 0, SEED, 53, 0, CHUNK, 20)]
-        t0 = time.perf_counter()
-        _, f2 = orc.col_binary(orc.ADD, orc.F64, f0, f1); _, f3 = orc.col_binary(orc.MUL, orc.F64, f2, f0)
-        _, i2 = orc.col_binary(orc.ADD, orc.I64, i0, i1); _, f4 = orc.col_cast(orc.I64, orc.F64, i2)
-        _, f5 = orc.col_binary(orc.DIV, orc.F64, f3, f1); _, f6 = orc.col_unary(orc.SIN, orc.F64, f5)
-        _, f7 = orc.col_binary(orc.ADD, orc.F64, f6, f4)
-        for op in (orc.SUM, orc.MAX, orc.MIN, orc.COUNT):
-            orc.aggregate(op, orc.I64, i2)
-        orc.aggregate(orc.SUM, orc.F64, f7); orc.aggregate(orc.COUNT, orc.F64, f7)
-        threads = 1
+
+        def step():
+            _, f2 = orc.col_binary(orc.ADD, orc.F64, f0, f1); _, f3 = orc.col_binary(orc.MUL, orc.F64, f2, f0)
+            _, i2 = orc.col_binary(orc.ADD, orc.I64, i0, i1); _, f4 = orc.col_cast(orc.I64, orc.F64, i2)
+            _, f5 = orc.col_binary(orc.DIV, orc.F64, f3, f1); _, f6 = orc.col_unary(orc.SIN, orc.F64, f5)
+            _, f7 = orc.col_binary(orc.ADD, orc.F64, f6, f4)
+            for op in (orc.SUM, orc.MAX, orc.MIN, orc.COUNT):
+                orc.aggregate(op, orc.I64, i2)
+            orc.aggregate(orc.SUM, orc.F64, f7); orc.aggregate(orc.COUNT, orc.F64, f7)
+    threads = 1
+    for _ in range(args.warmup):
+        step()
+    t0 = time.perf_counter()
+    for _ in range(args.steps):
+        step()
     dt = time.perf_counter() - t0
-    value = CHUNK / dt
-    line = {"impl": "reference", "metric": METRICS[cfg], "value": value, "unit": "rows/s", "n_gpus": args.gpus, "steps": 1, "warmup": 0,
-            "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "int64" if cfg == 3 else "f64",
+    value = CHUNK * args.steps / dt
+    line = {"impl": "reference", "metric": METRICS[cfg], "value": value, "unit": "rows/s", "n_gpus": args.gpus, "steps": args.steps,
+            "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
+            "dtype": "int64" if cfg == 3 else "f64",
             "data": "synthetic", "config": {"workload": WORKLOADS[cfg], "n_gpus": args.gpus, "scaling": args.scaling},
             "cpu_baseline": {"value": value, "unit": "rows/s", "cores": threads, "kind": "port",
                              "sample": "ONE 4e6-row chunk per column through the oracle, sequential over chunks on one thread as the reference's subtract/multiply/divide/sin/sum/max are; rows/s of the chunk"},

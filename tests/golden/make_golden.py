@@ -1,14 +1,13 @@
-"""Regenerates tests/golden/uk_cities.json from the reference's only data fixture.
+"""Rewrites tests/golden/uk_cities.json from the lat/lng columns it already stores (the reference's only data fixture).
 
-Run in the build container (the reference tree is not present on the GPU box):
     python tests/golden/make_golden.py
-The lat/lng columns come from /root/reference/test/data/uk_cities_with_headers.csv (37 rows); the
+The lat/lng columns are the 37 rows of the reference's test/data/uk_cities_with_headers.csv, kept in
+uk_cities.json itself, so the script needs nothing outside this repository; the
 `reference_asserts` block restates the numbers the reference's own tests assert on this fixture
 (src/dataframe.rs:803-808,835; src/lazyframe.rs:393-407).  `derived` values are produced by the CPU oracle
 (sequential folds, glibc sin) and are NOT asserted by the reference -- they pin the oracle against
 accidental change and give the GPU path a committed target.
 """
-import csv
 import json
 import os
 import sys
@@ -20,7 +19,7 @@ import numpy as np  # noqa: E402
 
 from oracle import pyoracle as orc  # noqa: E402
 
-SRC = "/root/reference/test/data/uk_cities_with_headers.csv"
+OUT = os.path.join(HERE, "uk_cities.json")
 
 
 class _Chunk:
@@ -29,11 +28,9 @@ class _Chunk:
 
 
 def main():
-    lat, lng = [], []
-    with open(SRC, newline="") as f:
-        for row in csv.DictReader(f):
-            lat.append(float(row["lat"]))
-            lng.append(float(row["lng"]))
+    with open(OUT) as f:
+        stored = json.load(f)
+    lat, lng = stored["lat"], stored["lng"]
     la, ln = np.array(lat), np.array(lng)
     _, added = orc.col_binary(orc.ADD, orc.F64, [_Chunk(la)], [_Chunk(ln)])
     _, sin_lat = orc.col_unary(orc.SIN, orc.F64, [_Chunk(la)])
@@ -57,7 +54,7 @@ def main():
             "min_lat": float(la.min()), "max_lat": float(la.max()),
         },
     }
-    with open(os.path.join(HERE, "uk_cities.json"), "w") as f:
+    with open(OUT, "w") as f:
         json.dump(out, f, indent=1)
     print("wrote uk_cities.json; sum(lat) =", float.fromhex(out["derived"]["sum_lat_hex"]))
 

@@ -17,8 +17,10 @@ def _gpu_count():
 
 
 def _sizes():
+    """Fleet sizes: 0 (Context.multi's "every visible GPU") and 1 on every machine, so the test ids do not depend on the machine
+    that collects them; 2, 3, 4 and 8 where the box has that many GPUs."""
     n = _gpu_count()
-    return [k for k in (1, 2, 3, 4, 8) if k <= n]
+    return [0, 1] + [k for k in (2, 3, 4, 8) if k <= n]
 
 
 def _chunks(rdf, name, seed, lens, null_frac):
@@ -38,12 +40,13 @@ def _chunks(rdf, name, seed, lens, null_frac):
 LENS = [100_001, 0, 1, 70_000, 64, 333_333, 4097]
 
 
-@pytest.fixture(scope="module", params=_sizes() or [0])
+@pytest.fixture(scope="module", params=_sizes())
 def fleet(request, rdf):
-    if not request.param:
+    n = _gpu_count()
+    if not n:
         pytest.skip("no GPU")
     ctx = rdf.Context.multi(request.param)
-    assert ctx.n_gpus == request.param
+    assert ctx.n_gpus == (request.param or n)
     yield ctx
     ctx.close()
 
