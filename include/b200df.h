@@ -22,6 +22,7 @@
  * Threads: a context may be called from several threads; calls on one context are serialised (a one-GPU context by a lock around each
  * entry, a multi-GPU context around each fan-out to its GPUs), so the reference's callers need no locking of their own -- but
  * bdf_destroy must not race with another call, and a column or future handle belongs to the thread that is using it.
+ * A column may be passed only to the context that made it; any other context returns BDF_INVALID.
  *
  * Error convention: every entry returns a bdf_status; BDF_OK == 0.  bdf_last_error() gives a
  * thread-local message.  No exception or abort crosses the ABI.  Mapping to the reference's errors:

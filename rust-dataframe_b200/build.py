@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libb200df.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["k_binary.cu", "k_unary.cu", "k_cast.cu", "k_reduce.cu", "k_filter.cu", "k_expr.cu", "k_sort.cu", "k_group.cu", "k_generate.cu", "runtime.cu", "ipc.cu", "comm.cu"]
+SOURCES = ["k_binary.cu", "k_unary.cu", "k_cast.cu", "k_reduce.cu", "k_filter.cu", "k_expr.cu", "k_sort.cu", "k_group.cu", "k_generate.cu", "runtime.cu", "fleet.cu", "ipc.cu", "comm.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 
@@ -42,7 +42,8 @@ def build_native(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(OBJ_DIR, exist_ok=True)
     nvcc = _nvcc()
     hdr_mtime = max(os.path.getmtime(os.path.join(CSRC, "common.cuh")), os.path.getmtime(os.path.join(CSRC, "comm.cuh")),
-                    os.path.getmtime(os.path.join(ROOT, "include", "b200df.h")), os.path.getmtime(__file__))
+                    os.path.getmtime(os.path.join(CSRC, "runtime.cuh")), os.path.getmtime(os.path.join(ROOT, "include", "b200df.h")),
+                    os.path.getmtime(__file__))
 
     def compile_one(src: str) -> str:
         obj = os.path.join(OBJ_DIR, src.replace(".cu", ".o"))

@@ -1,6 +1,6 @@
 // comm.cuh -- the one exchange step of the path (SURVEY.md 8(e)): the per-GPU partial aggregates are combined
 // with NCCL over NVLink / NVSwitch, enqueued on the stream that produced them (no host round trip between
-// the reducing kernel and the collective).  Implemented in comm.cu; used by runtime.cu only.
+// the reducing kernel and the collective).  Implemented in comm.cu; used by runtime.cu and fleet.cu only.
 //
 // Reference seam: the cross-chunk fold of AggregateFunctions::{sum,min,max,count}
 // (src/functions/aggregate.rs:12-31,70-93) -- chunks live on different GPUs here, so the fold over chunks

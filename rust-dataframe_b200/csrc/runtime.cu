@@ -12,30 +12,20 @@
 #include <cstdlib>
 #include <cstring>
 #include <condition_variable>
-#include <memory>
-#include <mutex>
 #include <new>
 #include <deque>
 #include <limits>
-#include <functional>
-#include <sched.h>
 #include <sys/mman.h>
-#include <string>
 #include <thread>
-#include <vector>
 
-#include "../../include/b200df.h"
-#include "common.cuh"
-#include "comm.cuh"
-
-using namespace bdf;
+#include "runtime.cuh"
 
 // ---------------------------------------------------------------------------------------------------
 // errors
 
-static thread_local std::string g_err;
+thread_local std::string g_err;
 
-static int fail(int status, const char* fmt, ...) {
+int fail(int status, const char* fmt, ...) {
     char buf[512];
     va_list ap;
     va_start(ap, fmt);
@@ -52,8 +42,6 @@ int set_error(int status, const char* msg) {   // for the host-only translation 
 }
 }  // namespace bdf
 
-static int cuda_status(cudaError_t e) { return e == cudaErrorMemoryAllocation ? BDF_OOM : BDF_CUDA; }
-
 // Set by the communicator layer (comm.cu reports NCCL failures as text + cudaErrorUnknown): turns the next
 // fail_cuda into BDF_NCCL.
 static thread_local std::string g_nccl_err;
@@ -66,80 +54,10 @@ static int fail_cuda(cudaError_t e, const char* what) {
     return fail(cuda_status(e), "%s failed: %s", what, cudaGetErrorString(e));
 }
 
-#define CK(call)                                                                                       \
-    do {                                                                                               \
-        cudaError_t _e = (call);                                                                       \
-        if (_e != cudaSuccess)                                                                         \
-            return fail(cuda_status(_e), "%s failed: %s (%s:%d)", #call, cudaGetErrorString(_e), __FILE__, __LINE__); \
-    } while (0)
-
-#define TRY(expr)                  \
-    do {                           \
-        int _st = (expr);          \
-        if (_st != BDF_OK) return _st; \
-    } while (0)
-
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // ---------------------------------------------------------------------------------------------------
 // objects
-
-struct Group {
-    int64_t begin, end;  // chunks [begin, end)
-    cudaEvent_t ev;      // chunks are complete in HBM once ev has fired
-};
-
-struct DevChunk {
-    char* values;
-    uint32_t* validity;  // nullptr = no bitmap
-    int64_t len;
-    int32_t bit_off;      // residual bit offset of the validity bitmap
-    int32_t val_bit_off;  // boolean columns only: residual bit offset of the VALUES bitmap
-};
-
-struct bdf_col {
-    int dtype = 0;
-    int64_t total_len = 0;
-    std::vector<DevChunk> chunks;
-    char* arena_values = nullptr;
-    char* arena_validity = nullptr;
-    uint32_t* d_warp_counts = nullptr;             // valid slots per warp per tile ([tile][8]), written by the producing kernel
-    int64_t tile_elems = 0;                        // tile size (elements) the producing kernel used
-    std::vector<int64_t> tile0;                    // column-global first tile of each chunk (n+1 entries)
-    bool counts_on_device = false;                 // d_warp_counts not yet folded into null_counts
-    std::vector<int64_t> null_counts;              // -1 = unknown
-    std::vector<Group> groups;
-    std::vector<uint32_t> dl_counts;               // staging of d_warp_counts during a split download
-    bdf_col* dl_tmp = nullptr;                     // re-aligned copy used by a split download of a sliced column
-    struct StagedCopy { void* dst; const void* src; size_t bytes; };
-    std::vector<StagedCopy> dl_staged;             // device->pageable-host copies carried out in download_finish
-    // A column of a multi-GPU context (bdf_init_multi): the logical chunks are cut into row ranges, each range lives as one
-    // chunk of a per-GPU sub-column.  Empty for the columns of a one-GPU context.
-    struct Piece { int kid; int64_t local; int64_t row0, rows; };   // rows [row0, row0 + rows) of a logical chunk = chunk `local` of fparts[kid]
-    std::vector<bdf_col*> fparts;                  // one sub-column per GPU (possibly without chunks)
-    std::vector<std::vector<Piece>> fmap;          // per logical chunk, in row order
-    std::vector<int64_t> flens;                    // logical chunk lengths
-};
-
-// Result of an aggregate that is still in flight (or done): a pinned slot + the event that guards it.
-struct bdf_future {
-    int n = 1;                   // number of aggregates the future carries (one per column of a multi-column call)
-    int fused = 1;               // which kernel produced the keys: 1 = k_binary AGG, 2 = k_reduce (see convert_agg)
-    int slot = 0;                // first index into h_agg: n records, or 2n ({AggDev, {rows, panics, chunks}}) when global
-    bool global = false;         // combined across the ranks of the communicator (comm.cuh)
-    int lslot = 0;               // global only: first index into d_local (the per-rank records the collective reads)
-    std::vector<int> dtypes;
-    std::vector<int64_t> rows;   // local rows per aggregate
-    std::vector<uint32_t> panics;  // local chunks that are empty or all-null (max/min .unwrap() would panic)
-    std::vector<uint32_t> chunks;  // local chunk count
-    cudaEvent_t ev = nullptr;
-    std::vector<bdf_future*> fparts;   // multi-GPU context: the per-GPU futures (every one yields the same, global, records)
-};
-
-struct ProfEntry {
-    bdf_launch_record rec;
-    cudaEvent_t e0, e1;
-};
 
 // Persistent host threads for the staged copies of PAGEABLE buffers (Arrow MutableBuffers, a mapped IPC file): a copy
 // is cut into 512 KiB jobs that the workers and the calling thread pull until it is done.  (Spawning threads per 8 MiB
@@ -209,73 +127,35 @@ class CopyPool {
     bool stop_ = false, populate_ = false;
 };
 
-struct bdf_ctx {
-    int device = 0;
-    int sm_count = 0, cc_major = 0, cc_minor = 0;
-    size_t hbm_bytes = 0;
-    cudaStream_t s_compute = nullptr, s_h2d = nullptr, s_d2h = nullptr;
-    cudaStream_t s_desc = nullptr;  // descriptor copies: run ahead of the compute stream, off its critical path
-    cudaStream_t s_fin = nullptr;   // k_finish of fused aggregates: overlaps the next operator
-    std::mutex mu;
-    // pinned staging: descriptor ring + small result area
-    char* ring = nullptr;           // pinned host side of the descriptor ring
-    char* dring = nullptr;          // device side, same offsets
-    size_t ring_cap = 0, ring_head = 0;
-    std::vector<cudaEvent_t> ev_pool;  // recycled cudaEventDisableTiming events
-    AggDev* h_agg = nullptr;        // pinned + device-mapped: kernels write results straight into it
-    AggDev* h_agg_dev = nullptr;    // device-side address of h_agg
-    int* h_flag = nullptr;          // pinned
-    unsigned long long* h_sort_agree = nullptr;   // pinned: OR and AND of the sort keys of one criterion
-    int64_t last_sort_passes = 0;
-    // device scratch
-    AggDev* d_partials = nullptr;       // per-CTA partials of k_reduce (compute stream only)
-    size_t red_part_cap = 0;
-    AggDev* d_stage2 = nullptr;         // k_finish staging for the k_reduce path
-    AggDev* d_stage_many = nullptr;     // k_finish_many staging (kFinishMany x sm_count) and tickets, allocated on first use
-    unsigned int* d_tickets_many = nullptr;
-    unsigned int* d_ticket = nullptr;   // k_finish tickets: [0] reduce path (compute stream), [1] fused aggregates (finish stream)
-    AggDev* d_stage = nullptr;          // k_finish per-CTA staging, sm_count entries
-    int* d_flag = nullptr;
-    int fut_next = 0;                   // ring cursor over the future half of h_agg
-    struct PartBuf { AggDev* p = nullptr; size_t cap = 0; cudaEvent_t done = nullptr; bool used = false; } part[3];
-    int part_next = 0;                  // per-tile partials of fused aggregates: 3 persistent buffers in rotation
-    // staging for PAGEABLE host buffers: pinned slots filled/drained by a few host threads while the DMA of the
-    // previous slot is in flight (cudaMemcpyAsync straight from pageable memory is a single-threaded driver copy)
-    struct StageSlot { char* p = nullptr; cudaEvent_t ev = nullptr; bool busy = false; };
-    std::vector<StageSlot> stage;
-    int stage_next = 0;
-    int copy_threads = 8;
-    std::unique_ptr<CopyPool> pool;
-    cudaEvent_t ev_tmp = nullptr, ev_t0 = nullptr, ev_t1 = nullptr;
-    void* flush_buf = nullptr;
-    size_t flush_bytes = 0;
-    size_t pipeline_bytes = (size_t)32 << 20;
-    bool profiling = false;
-    std::vector<ProfEntry> prof;
-    std::vector<cudaEvent_t> prof_pool;   // recycled timing events
-    int64_t launches = 0;
-    // multi-GPU: the communicator this context is a rank of (nullptr = a lone GPU) -- comm.cuh
-    Comm* comm = nullptr;
-    bool collective = true;             // aggregates are combined across the ranks (every rank makes the same calls)
-    AggDev* d_local = nullptr;          // per-rank aggregate records awaiting their collective (ring of kAggSlots)
-    int local_next = 0;
-    int64_t collectives = 0;            // grouped NCCL calls enqueued since the communicator was attached
-    struct Fleet* fleet = nullptr;      // non-null: this is a multi-GPU context (bdf_init_multi); it owns no device itself
-};
+bdf_ctx::bdf_ctx() = default;
+bdf_ctx::~bdf_ctx() = default;
 
 static constexpr int kAggSlots = 4096;
 
 // ---------------------------------------------------------------------------------------------------
 // small helpers
 
-static constexpr int kBool = 10;  // BDF_BOOL: bit-packed boolean column (N2)
-
 static inline size_t value_bytes(int dtype, int64_t len, int bit_off) {
     return dtype == kBool ? (size_t)((len + bit_off + 7) / 8) : (size_t)len * dtype_width(dtype);
 }
 
-static int check_dtype(int t) {
-    if (t < 0 || t >= BDF_NTYPES) return fail(BDF_INVALID, "invalid dtype %d", t);
+// The first check of every entry that takes columns: a context, and columns that context made.  Reads only what is fixed
+// when a column is made, so it runs before the context's lock is taken.
+static int check_cols(const bdf_ctx* c, int64_t n, const bdf_col* const* cols) {
+    if (!c) return fail(BDF_INVALID, "null context");
+    for (int64_t i = 0; i < n; i++) {
+        if (!cols[i]) return fail(BDF_INVALID, "null argument");
+        if (cols[i]->owner != c) return fail(BDF_INVALID, "a column may only be passed to the context that made it");
+    }
+    return BDF_OK;
+}
+static int check_cols(const bdf_ctx* c, std::initializer_list<const bdf_col*> cols) { return check_cols(c, (int64_t)cols.size(), cols.begin()); }
+
+// Host chunks: a count, and views with sane lengths and offsets.
+static int check_views(int64_t n, const bdf_view* v) {
+    if (n < 0 || (n && !v)) return fail(BDF_INVALID, "bad arguments");
+    for (int64_t i = 0; i < n; i++)
+        if (v[i].len < 0 || v[i].offset < 0 || (v[i].len > 0 && !v[i].values)) return fail(BDF_INVALID, "bad view %lld", (long long)i);
     return BDF_OK;
 }
 
@@ -365,6 +245,7 @@ static int col_alloc(bdf_ctx* c, int dtype, const std::vector<ChunkPlan>& plan, 
                      int64_t tile_elems, bdf_col** out) {
     bdf_col* col = new (std::nothrow) bdf_col();
     if (!col) return fail(BDF_OOM, "host allocation failed");
+    col->owner = c;
     col->dtype = dtype;
     const int w = dtype_width(dtype);
     const size_t n = plan.size();
@@ -640,7 +521,6 @@ static int upload_many(bdf_ctx* c, const std::vector<UploadSpec>& specs, bool as
         std::vector<int32_t> offs((size_t)s.n);
         for (int64_t i = 0; i < s.n; i++) {
             const bdf_view& v = s.views[i];
-            if (v.len < 0 || v.offset < 0 || (v.len > 0 && !v.values)) { cleanup(); return fail(BDF_INVALID, "bad view %lld", (long long)i); }
             plan[i] = {v.len, v.validity != nullptr};
             offs[i] = (int32_t)(v.offset & 7);
         }
@@ -924,7 +804,6 @@ static int map_dev(bdf_ctx* c, bool is_cast, int op_or_to, const bdf_col* in, bd
     if (from == kBool) return fail(BDF_UNSUPPORTED, "numeric function on a boolean column");
     if (is_cast) {
         to = op_or_to;
-        TRY(check_dtype(to));
     } else {
         const int op = op_or_to;
         if (op < 0 || op >= BDF_NUNARY) return fail(BDF_INVALID, "invalid unary op %d", op);
@@ -1146,11 +1025,8 @@ static int count_panic_chunks(bdf_ctx* c, bdf_col* col, uint32_t* out) {
 // communicator -- ONE grouped collective for all of them.  need_counts: also evaluate the would-panic rule (may
 // synchronise to learn null counts of uploaded columns).
 static int aggregate_many_dev_async(bdf_ctx* c, int n_cols, bdf_col* const* cols, bool need_counts, bdf_future** fut) {
-    if (n_cols < 1 || n_cols > kCommMaxCols) return fail(BDF_INVALID, "an aggregate call takes 1..%d columns", kCommMaxCols);
-    for (int k = 0; k < n_cols; k++) {
-        if (!cols[k]) return fail(BDF_INVALID, "null column");
+    for (int k = 0; k < n_cols; k++)
         if (cols[k]->dtype == kBool) return fail(BDF_UNSUPPORTED, "aggregate of a boolean column");
-    }
     std::vector<uint32_t> panics((size_t)n_cols, 0u);
     if (need_counts)
         for (int k = 0; k < n_cols; k++) TRY(count_panic_chunks(c, cols[k], &panics[k]));
@@ -1174,10 +1050,6 @@ static int aggregate_many_dev_async(bdf_ctx* c, int n_cols, bdf_col* const* cols
     }
     *fut = f;
     return BDF_OK;
-}
-
-static int aggregate_all_dev_async(bdf_ctx* c, bdf_col* col, bdf_future** fut) {
-    return aggregate_many_dev_async(c, 1, &col, false, fut);
 }
 
 // Waits for the future, converts its n records into out[0..n) and consumes it.
@@ -1222,7 +1094,6 @@ static int count_global(bdf_ctx* c, int64_t* total) {
 }
 
 static int aggregate_dev(bdf_ctx* c, int op, bdf_col* col, void* out_scalar, int32_t* is_some) {
-    if (op < 0 || op >= BDF_NAGG) return fail(BDF_INVALID, "invalid aggregate op %d", op);
     const int dtype = col->dtype;
     const int w = dtype_width(dtype);
     if (op == BDF_COUNT) {  // metadata only, as in the reference (aggregate.rs:70-80)
@@ -1234,8 +1105,6 @@ static int aggregate_dev(bdf_ctx* c, int op, bdf_col* col, void* out_scalar, int
         *is_some = 1;
         return BDF_OK;
     }
-    if ((op == BDF_MIN || op == BDF_MAX) && dtype_is_float(dtype))
-        return fail(BDF_UNSUPPORTED, "min/max need T::Native: Ord (integers only)");
     bdf_agg4 a;
     TRY(aggregate_all_dev(c, col, op != BDF_SUM, &a));
     if (op == BDF_SUM) {
@@ -1548,20 +1417,9 @@ static int expr_prepare(int n_inputs, const int* in_dtypes, int n_nodes, const b
     }
 }
 
-// out == nullptr (only with fut): aggregate only, the result column is never written.
-static int expr_dev(bdf_ctx* c, int n_inputs, const bdf_col* const* inputs, int n_nodes, const bdf_expr_node* nodes, bdf_col** out,
-                    bdf_future** fut = nullptr) {
-    if (!inputs) return fail(BDF_INVALID, "null argument");
-    int in_dtypes[8] = {0};
-    for (int i = 0; i < n_inputs && i < 8; i++) {
-        if (!inputs[i]) return fail(BDF_INVALID, "null input column");
-        in_dtypes[i] = inputs[i]->dtype;
-    }
-    alignas(8) unsigned char prog[256];
-    bool has_div = false;
-    TRY(expr_prepare(n_inputs, in_dtypes, n_nodes, nodes, prog, &has_div));
-    for (int i = 0; i < n_inputs; i++)
-        if (!inputs[i]) return fail(BDF_INVALID, "null input column");
+// prog: the program expr_prepare compiled.  out == nullptr (only with fut): aggregate only, the result column is never written.
+static int expr_dev(bdf_ctx* c, int n_inputs, const bdf_col* const* inputs, const unsigned char* prog, bool has_div, bdf_col** out,
+                    bdf_future** fut) {
     int64_t n = (int64_t)inputs[0]->chunks.size();
     for (int i = 0; i < n_inputs; i++) {
         n = std::min<int64_t>(n, (int64_t)inputs[i]->chunks.size());
@@ -1699,7 +1557,6 @@ static int sort_table(bdf_ctx* c, const bdf_col* col, void** dev, int* n_chunks,
 static int sort_indices_dev(bdf_ctx* c, int n_keys, const bdf_sort_key* keys, bdf_col** out) {
     if (n_keys < 1) return fail(BDF_INVALID, "Sort criteria cannot be empty");
     for (int k = 0; k < n_keys; k++) {
-        if (!keys[k].column) return fail(BDF_INVALID, "null sort column");
         const int dt = keys[k].column->dtype;
         if (dt < 0 || dt >= BDF_NTYPES) return fail(BDF_UNSUPPORTED, "sort criteria must be numeric columns");
         if (keys[k].column->total_len != keys[0].column->total_len) return fail(BDF_LENGTH_MISMATCH, "sort columns have different lengths");
@@ -1811,9 +1668,7 @@ size_t group_big_scratch_bytes(long long n_rows);
 static int group_aggregate_dev(bdf_ctx* c, const bdf_col* key, int n_values, const bdf_col* const* values, bdf_col** out_keys,
                                bdf_group_out* outs, int64_t* n_groups_out) {
     if (key->dtype < 0 || key->dtype >= BDF_NTYPES) return fail(BDF_UNSUPPORTED, "the group key must be a numeric column");
-    if (n_values < 0 || n_values > 64) return fail(BDF_INVALID, "0..64 value columns");
     for (int j = 0; j < n_values; j++) {
-        if (!values[j]) return fail(BDF_INVALID, "null value column");
         if (values[j]->dtype < 0 || values[j]->dtype >= BDF_NTYPES) return fail(BDF_UNSUPPORTED, "aggregated columns must be numeric");
         if (values[j]->total_len != key->total_len) return fail(BDF_LENGTH_MISMATCH, "key and value columns have different lengths");
     }
@@ -1908,586 +1763,33 @@ static int group_aggregate_dev(bdf_ctx* c, const bdf_col* key, int n_values, con
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Multi-GPU context (bdf_init_multi): ONE process, every GPU of the box.  The library owns the sharding that the
-// reference leaves to rayon (par_iter over chunks, src/functions/scalar.rs:28-31,99-102): the rows of a call are cut into
-// one contiguous range per GPU (cuts on 64-row boundaries inside a chunk, so a piece is a zero-copy Arrow slice whose
-// validity starts on a byte boundary), every GPU runs the ordinary one-GPU path on its pieces -- its own PCIe link, its
-// own staging threads -- and aggregates are combined by the grouped ncclAllReduce of comm.cu (ncclCommInitAll).
-// A fleet context owns no device; its "kids" are complete one-GPU contexts driven by one persistent host thread each
-// (a blocking collective must be entered by all ranks at once, and uploads of different GPUs should overlap).
-
-struct Fleet {
-    std::vector<bdf_ctx*> kids;
-    struct Worker {
-        std::thread th;
-        std::mutex m;
-        std::condition_variable cv;
-        std::function<int()> job;
-        bool has_job = false, done = false, stop = false;
-        int status = BDF_OK;
-        std::string err;
-    };
-    std::vector<std::unique_ptr<Worker>> workers;
-    std::mutex run_mu;   // one fan-out at a time: two caller threads must not interleave their jobs (or the order of the kids' collectives)
-};
-
-static void fleet_worker_main(Fleet::Worker* w, int device) {
-    // run near the GPU: host<->device copies and the staging threads this thread creates stay on the GPU's NUMA node
-    char bus[32];
-    if (cudaDeviceGetPCIBusId(bus, sizeof bus, device) == cudaSuccess) {
-        for (char* p = bus; *p; p++) *p = (char)tolower(*p);
-        const std::string base = std::string("/sys/bus/pci/devices/") + bus + "/numa_node";
-        int node = -1;
-        if (FILE* f = fopen(base.c_str(), "r")) { if (fscanf(f, "%d", &node) != 1) node = -1; fclose(f); }
-        if (node >= 0) {
-            const std::string cl = "/sys/devices/system/node/node" + std::to_string(node) + "/cpulist";
-            if (FILE* f = fopen(cl.c_str(), "r")) {
-                char buf[4096];
-                if (fgets(buf, sizeof buf, f)) {
-                    cpu_set_t set, cur; CPU_ZERO(&set);
-                    int n = 0;
-                    for (char* tok = strtok(buf, ",\n"); tok; tok = strtok(nullptr, ",\n")) {
-                        int lo, hi;
-                        if (sscanf(tok, "%d-%d", &lo, &hi) == 2) { for (int cpu = lo; cpu <= hi && cpu < CPU_SETSIZE; cpu++) { CPU_SET(cpu, &set); n++; } }
-                        else if (sscanf(tok, "%d", &lo) == 1 && lo < CPU_SETSIZE) { CPU_SET(lo, &set); n++; }
-                    }
-                    if (n && sched_getaffinity(0, sizeof cur, &cur) == 0) {
-                        CPU_AND(&set, &set, &cur);
-                        if (CPU_COUNT(&set) > 0) sched_setaffinity(0, sizeof set, &set);
-                    }
-                }
-                fclose(f);
-            }
-        }
-    }
-    cudaGetLastError();
-    std::unique_lock<std::mutex> lk(w->m);
-    for (;;) {
-        w->cv.wait(lk, [w] { return w->has_job || w->stop; });
-        if (w->stop) return;
-        std::function<int()> job = std::move(w->job);
-        w->has_job = false;
-        lk.unlock();
-        g_err.clear();
-        int st;
-        try { st = job(); } catch (...) { st = fail(BDF_INVALID, "internal error in a fleet worker"); }
-        lk.lock();
-        w->status = st;
-        w->err = g_err;
-        w->done = true;
-        w->cv.notify_all();
-    }
-}
-
-// Run fn(k) for every kid, each on its own thread, and wait.  The first failing status (lowest kid) is returned with its message.
-static int fleet_run(Fleet* f, const std::function<int(int)>& fn) {
-    std::lock_guard<std::mutex> one_at_a_time(f->run_mu);   // the jobs run on the workers and never fan out themselves: no recursion
-    const int n = (int)f->kids.size();
-    for (int k = 0; k < n; k++) {
-        Fleet::Worker* w = f->workers[k].get();
-        std::lock_guard<std::mutex> g(w->m);
-        w->job = [&fn, k] { return fn(k); };
-        w->has_job = true; w->done = false;
-        w->cv.notify_all();
-    }
-    int status = BDF_OK;
-    std::string err;
-    for (int k = 0; k < n; k++) {
-        Fleet::Worker* w = f->workers[k].get();
-        std::unique_lock<std::mutex> lk(w->m);
-        w->cv.wait(lk, [w] { return w->done; });
-        if (w->status != BDF_OK && status == BDF_OK) { status = w->status; err = w->err; }
-    }
-    if (status != BDF_OK) g_err = err;
-    return status;
-}
-
-static bool is_fleet_col(const bdf_col* col) { return col && !col->fparts.empty(); }
-
-// Cut the rows of the logical chunks into one contiguous range per kid (balanced by rows; cuts inside a chunk are
-// multiples of 64 rows).  Returns the pieces per logical chunk; `local` numbers a kid's pieces in order.
-static std::vector<std::vector<bdf_col::Piece>> fleet_plan(const std::vector<int64_t>& lens, int n_kids) {
-    const size_t n = lens.size();
-    int64_t total = 0;
-    std::vector<int64_t> start(n + 1, 0);
-    for (size_t i = 0; i < n; i++) { start[i] = total; total += lens[i]; }
-    start[n] = total;
-    auto snap = [&](int64_t g) {   // a global cut -> an aligned row of the chunk it falls into
-        if (g <= 0) return (int64_t)0;
-        if (g >= total) return total;
-        size_t i = (size_t)(std::upper_bound(start.begin(), start.begin() + (ptrdiff_t)n, g) - start.begin()) - 1;
-        return start[i] + (g - start[i]) / 64 * 64;
-    };
-    std::vector<int64_t> cut((size_t)n_kids + 1);
-    for (int k = 0; k <= n_kids; k++) cut[k] = snap((int64_t)((__int128)total * k / n_kids));
-    cut[n_kids] = total;
-    std::vector<std::vector<bdf_col::Piece>> map(n);
-    std::vector<int64_t> next_local((size_t)n_kids, 0);
-    for (size_t i = 0; i < n; i++)
-        for (int k = 0; k < n_kids; k++) {
-            const int64_t b = std::max(cut[k], start[i]), e = std::min(cut[k + 1], start[i] + lens[i]);
-            if (e > b) map[i].push_back(bdf_col::Piece{k, next_local[k]++, b - start[i], e - b});
-        }
-    // an empty logical chunk still needs a home (it keeps the chunk structure and the reference's panic rule intact)
-    for (size_t i = 0; i < n; i++)
-        if (lens[i] == 0) map[i].push_back(bdf_col::Piece{(int)(i % (size_t)n_kids), next_local[i % (size_t)n_kids]++, 0, 0});
-    return map;
-}
-
-// The host views of kid k under a plan (zero-copy slices of the caller's chunks), in the kid's local chunk order.
-static std::vector<bdf_view> fleet_views(const std::vector<std::vector<bdf_col::Piece>>& map, int n_kids, int kid, const bdf_view* in) {
-    std::vector<std::pair<int64_t, bdf_view>> mine;
-    for (size_t i = 0; i < map.size(); i++)
-        for (const auto& pc : map[i])
-            if (pc.kid == kid) {
-                bdf_view v = in[i];
-                v.offset += pc.row0;
-                v.len = pc.rows;
-                if (!(pc.row0 == 0 && pc.rows == in[i].len)) v.null_count = v.validity ? -1 : 0;   // a proper slice: unknown
-                mine.push_back({pc.local, v});
-            }
-    (void)n_kids;
-    std::sort(mine.begin(), mine.end(), [](const auto& a, const auto& b) { return a.first < b.first; });
-    std::vector<bdf_view> out;
-    for (auto& m : mine) out.push_back(m.second);
-    return out;
-}
-
-static std::vector<bdf_out> fleet_outs(const std::vector<std::vector<bdf_col::Piece>>& map, int kid, int out_dtype, const bdf_out* out) {
-    std::vector<std::pair<int64_t, bdf_out>> mine;
-    const int w = out_dtype == kBool ? 0 : dtype_width(out_dtype);
-    for (size_t i = 0; i < map.size(); i++)
-        for (const auto& pc : map[i])
-            if (pc.kid == kid) {
-                bdf_out o = out[i];
-                if (o.values) o.values = (char*)o.values + (out_dtype == kBool ? pc.row0 / 8 : pc.row0 * w);
-                if (o.validity) o.validity = o.validity + pc.row0 / 8;   // row0 is a multiple of 64
-                o.len = pc.rows;
-                mine.push_back({pc.local, o});
-            }
-    std::sort(mine.begin(), mine.end(), [](const auto& a, const auto& b) { return a.first < b.first; });
-    std::vector<bdf_out> res;
-    for (auto& m : mine) res.push_back(m.second);
-    return res;
-}
-
-// Fold the kids' per-piece results back into the caller's per-chunk bdf_out entries.
-static void fleet_merge_outs(const std::vector<std::vector<bdf_col::Piece>>& map, const std::vector<std::vector<bdf_out>>& kid_outs,
-                             const std::vector<int64_t>& lens, bdf_out* out) {
-    for (size_t i = 0; i < map.size(); i++) {
-        int64_t nulls = 0;
-        int32_t hv = 0;
-        for (const auto& pc : map[i]) {
-            const bdf_out& o = kid_outs[(size_t)pc.kid][(size_t)pc.local];
-            nulls += o.null_count;
-            hv |= o.has_validity;
-        }
-        out[i].len = lens[i];
-        out[i].null_count = nulls;
-        out[i].has_validity = hv;
-    }
-}
-
-static bool fleet_same_map(const bdf_col* a, const bdf_col* b, int64_t n) {
-    if ((int64_t)a->fmap.size() < n || (int64_t)b->fmap.size() < n) return false;
-    for (int64_t i = 0; i < n; i++) {
-        if (a->fmap[i].size() != b->fmap[i].size()) return false;
-        for (size_t j = 0; j < a->fmap[i].size(); j++) {
-            const auto &x = a->fmap[i][j], &y = b->fmap[i][j];
-            if (x.kid != y.kid || x.local != y.local || x.row0 != y.row0 || x.rows != y.rows) return false;
-        }
-    }
-    return true;
-}
-
-static bdf_col* fleet_col_new(int dtype, int n_kids) {
-    bdf_col* col = new (std::nothrow) bdf_col();
-    if (!col) return nullptr;
-    col->dtype = dtype;
-    col->fparts.assign((size_t)n_kids, nullptr);
-    return col;
-}
-
-static void fleet_col_free(Fleet* f, bdf_col* col) {
-    if (!col) return;
-    for (size_t k = 0; k < col->fparts.size(); k++)
-        if (col->fparts[k]) bdf_col_free(f->kids[k], col->fparts[k]);
-    delete col;
-}
-
-// A result column with the logical structure of `like` (elementwise operators keep it), parts filled by the kids.
-static bdf_col* fleet_col_like(const bdf_col* like, int dtype, int n_kids, int64_t n_chunks) {
-    bdf_col* col = fleet_col_new(dtype, n_kids);
-    if (!col) return nullptr;
-    col->fmap.assign(like->fmap.begin(), like->fmap.begin() + (ptrdiff_t)n_chunks);
-    col->flens.assign(like->flens.begin(), like->flens.begin() + (ptrdiff_t)n_chunks);
-    col->total_len = 0;
-    for (int64_t v : col->flens) col->total_len += v;
-    return col;
-}
-
-static int fleet_upload_many(bdf_ctx* c, int64_t n_cols, const int32_t* dtypes, const int64_t* n_chunks, const bdf_view* const* in, int flags, bdf_col** out) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    // all columns of one call share ONE plan when their chunk lengths agree (a RecordBatch list), so that operators over them line up
-    std::vector<bdf_col*> cols((size_t)n_cols, nullptr);
-    std::vector<std::vector<std::vector<bdf_view>>> views((size_t)n_cols);
-    for (int64_t j = 0; j < n_cols; j++) {
-        std::vector<int64_t> lens((size_t)n_chunks[j]);
-        for (int64_t i = 0; i < n_chunks[j]; i++) {
-            if (in[j][i].len < 0 || in[j][i].offset < 0) { for (auto* x : cols) fleet_col_free(f, x); return fail(BDF_INVALID, "bad view %lld", (long long)i); }
-            lens[i] = in[j][i].len;
-        }
-        cols[j] = fleet_col_new(dtypes[j], nk);
-        if (!cols[j]) { for (auto* x : cols) fleet_col_free(f, x); return fail(BDF_OOM, "host allocation failed"); }
-        cols[j]->fmap = fleet_plan(lens, nk);
-        cols[j]->flens = lens;
-        for (int64_t v : lens) cols[j]->total_len += v;
-        views[j].resize((size_t)nk);
-        for (int k = 0; k < nk; k++) views[j][k] = fleet_views(cols[j]->fmap, nk, k, in[j]);
-    }
-    int st = fleet_run(f, [&](int k) {
-        std::vector<int32_t> dt((size_t)n_cols);
-        std::vector<int64_t> cnt((size_t)n_cols);
-        std::vector<const bdf_view*> ptr((size_t)n_cols);
-        std::vector<bdf_col*> res((size_t)n_cols, nullptr);
-        for (int64_t j = 0; j < n_cols; j++) { dt[j] = dtypes[j]; cnt[j] = (int64_t)views[j][k].size(); ptr[j] = views[j][k].data(); }
-        int s2 = bdf_upload_many(f->kids[k], n_cols, dt.data(), cnt.data(), ptr.data(), flags, res.data());
-        for (int64_t j = 0; j < n_cols; j++) cols[j]->fparts[k] = res[j];
-        return s2;
-    });
-    if (st != BDF_OK) { const std::string keep = g_err; for (auto* x : cols) fleet_col_free(f, x); g_err = keep; return st; }
-    for (int64_t j = 0; j < n_cols; j++) out[j] = cols[j];
-    return BDF_OK;
-}
-
-static int fleet_download(bdf_ctx* c, const bdf_col* col, bdf_out* out, int phase /* 0 both, 1 begin, 2 end */) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    const int64_t n = (int64_t)col->fmap.size();
-    for (int64_t i = 0; i < n; i++)
-        if (out[i].len != col->flens[i]) return fail(BDF_INVALID, "output chunk %lld has capacity %lld, result has %lld rows", (long long)i, (long long)out[i].len, (long long)col->flens[i]);
-    std::vector<std::vector<bdf_out>> kouts((size_t)nk);
-    for (int k = 0; k < nk; k++) kouts[k] = fleet_outs(col->fmap, k, col->dtype, out);
-    int st = fleet_run(f, [&](int k) {
-        bdf_out dummy{};
-        bdf_out* o = kouts[k].empty() ? &dummy : kouts[k].data();
-        if (phase == 1) return bdf_download_begin(f->kids[k], col->fparts[k], o);
-        if (phase == 2) return bdf_download_end(f->kids[k], col->fparts[k], o);
-        return bdf_download(f->kids[k], col->fparts[k], o);
-    });
-    if (st != BDF_OK) return st;
-    if (phase != 1) fleet_merge_outs(col->fmap, kouts, col->flens, out);
-    return BDF_OK;
-}
-
-// One elementwise operator over fleet columns: `call(k, parts of the inputs on kid k, &result part)`.
-static int fleet_map(bdf_ctx* c, int out_dtype, std::initializer_list<const bdf_col*> inputs, bdf_col** out,
-                     const std::function<int(int, bdf_col**)>& call) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    const bdf_col* first = *inputs.begin();
-    int64_t n = (int64_t)first->fmap.size();
-    for (const bdf_col* col : inputs) {
-        if (!is_fleet_col(col)) return fail(BDF_INVALID, "a column of a one-GPU context was passed to a multi-GPU context");
-        n = std::min<int64_t>(n, (int64_t)col->fmap.size());   // zip()
-    }
-    for (const bdf_col* col : inputs) {
-        for (int64_t i = 0; i < n; i++)
-            if (col->flens[i] != first->flens[i]) return fail(BDF_LENGTH_MISMATCH, "Cannot perform math operation on arrays of different length");
-        if (!fleet_same_map(first, col, n)) return fail(BDF_INVALID, "the columns are sharded differently over the GPUs (upload them in one bdf_upload_many call)");
-        if (col->fmap.size() != first->fmap.size()) return fail(BDF_UNSUPPORTED, "columns with different numbers of chunks on a multi-GPU context");
-    }
-    bdf_col* o = fleet_col_like(first, out_dtype, nk, n);
-    if (!o) return fail(BDF_OOM, "host allocation failed");
-    int st = fleet_run(f, [&](int k) { return call(k, &o->fparts[k]); });
-    if (st != BDF_OK) { const std::string keep = g_err; fleet_col_free(f, o); g_err = keep; return st; }
-    *out = o;
-    return BDF_OK;
-}
-
-static bdf_future* fleet_future_new(int n_kids) {
-    bdf_future* fu = new (std::nothrow) bdf_future();
-    if (fu) fu->fparts.assign((size_t)n_kids, nullptr);
-    return fu;
-}
-
-static int fleet_future_wait(bdf_ctx* c, bdf_future* fu, bdf_agg4* out) {
-    Fleet* f = c->fleet;
-    const int n = fu->n;
-    std::vector<std::vector<bdf_agg4>> res(f->kids.size(), std::vector<bdf_agg4>((size_t)std::max(n, 1)));
-    int st = fleet_run(f, [&](int k) { return fu->fparts[k] ? bdf_future_wait(f->kids[k], fu->fparts[k], res[k].data()) : BDF_OK; });
-    if (st == BDF_OK && out) for (int i = 0; i < n; i++) out[i] = res[0][i];   // every rank holds the same global records
-    delete fu;
-    return st;
-}
-
-// Aggregates of n columns: every kid reduces its parts, the collective inside the kids' call makes the result global.
-static int fleet_aggregate_many(bdf_ctx* c, int32_t n_cols, const bdf_col* const* cols, bdf_future** fut) {
-    Fleet* f = c->fleet;
-    if (n_cols < 1 || n_cols > kCommMaxCols) return fail(BDF_INVALID, "an aggregate call takes 1..%d columns", kCommMaxCols);
-    for (int32_t j = 0; j < n_cols; j++)
-        if (!is_fleet_col(cols[j])) return fail(BDF_INVALID, "a column of a one-GPU context was passed to a multi-GPU context");
-    bdf_future* fu = fleet_future_new((int)f->kids.size());
-    if (!fu) return fail(BDF_OOM, "host allocation failed");
-    fu->n = n_cols;
-    int st = fleet_run(f, [&](int k) {
-        std::vector<const bdf_col*> parts((size_t)n_cols);
-        for (int32_t j = 0; j < n_cols; j++) parts[j] = cols[j]->fparts[k];
-        return bdf_aggregate_all_many_dev_async(f->kids[k], n_cols, parts.data(), &fu->fparts[k]);
-    });
-    if (st != BDF_OK) { const std::string keep = g_err; fleet_future_wait(c, fu, nullptr); g_err = keep; return st; }
-    *fut = fu;
-    return BDF_OK;
-}
-
-// Logical chunks of a fleet column without a valid slot (empty or all-null): the reference's max/min unwrap() a None there.
-// Evaluated over the caller's chunks -- a piece may be all-null while its chunk is not.
-static int fleet_panic_chunks(bdf_ctx* c, const bdf_col* col, int* out) {
-    Fleet* f = c->fleet;
-    const size_t n = col->fmap.size();
-    std::vector<int64_t> valid(n, 0);
-    std::mutex m;
-    int st = fleet_run(f, [&](int k) {
-        for (size_t i = 0; i < n; i++)
-            for (const auto& pc : col->fmap[i])
-                if (pc.kid == k) {
-                    int64_t len = 0, nulls = 0; int32_t hv = 0;
-                    int s2 = bdf_col_chunk_info(f->kids[k], col->fparts[k], pc.local, &len, &nulls, &hv);
-                    if (s2 != BDF_OK) return s2;
-                    std::lock_guard<std::mutex> g(m);
-                    valid[i] += len - (hv ? nulls : 0);
-                }
-        return (int)BDF_OK;
-    });
-    if (st != BDF_OK) return st;
-    int k = 0;
-    for (size_t i = 0; i < n; i++) if (valid[i] == 0) k++;
-    *out = k;
-    return BDF_OK;
-}
-
-static int fleet_aggregate_dev(bdf_ctx* c, int op, const bdf_col* col, void* out_scalar, int32_t* is_some) {
-    if (op < 0 || op >= BDF_NAGG) return fail(BDF_INVALID, "invalid aggregate op %d", op);
-    if (!is_fleet_col(col)) return fail(BDF_INVALID, "a column of a one-GPU context was passed to a multi-GPU context");
-    const int dtype = col->dtype;
-    if ((op == BDF_MIN || op == BDF_MAX) && dtype_is_float(dtype)) return fail(BDF_UNSUPPORTED, "min/max need T::Native: Ord (integers only)");
-    if (dtype == kBool) return fail(BDF_UNSUPPORTED, "aggregate of a boolean column");
-    bdf_future* fu = nullptr;
-    TRY(fleet_aggregate_many(c, 1, &col, &fu));
-    bdf_agg4 a;
-    TRY(fleet_future_wait(c, fu, &a));
-    const int w = dtype_width(dtype);
-    if (op == BDF_COUNT) { *(int64_t*)out_scalar = a.count; *is_some = 1; return BDF_OK; }
-    if (op == BDF_SUM) { memcpy(out_scalar, &a.sum, (size_t)w); *is_some = 1; return BDF_OK; }
-    int panics = 0;
-    TRY(fleet_panic_chunks(c, col, &panics));
-    if (panics) return fail(BDF_WOULD_PANIC, "max/min on an empty or all-null chunk: the reference unwraps None");
-    *is_some = col->fmap.empty() ? 0 : 1;
-    if (*is_some) memcpy(out_scalar, op == BDF_MIN ? &a.min : &a.max, (size_t)w);
-    return BDF_OK;
-}
-
-static int fleet_aggregate_all_blocking(bdf_ctx* c, int32_t n_cols, const bdf_col* const* cols, bdf_agg4* out) {
-    bdf_future* fu = nullptr;
-    TRY(fleet_aggregate_many(c, n_cols, cols, &fu));
-    TRY(fleet_future_wait(c, fu, out));
-    for (int32_t j = 0; j < n_cols; j++) {
-        int panics = 0;
-        TRY(fleet_panic_chunks(c, cols[j], &panics));
-        out[j].would_panic = panics != 0;
-        out[j].n_chunks = (int64_t)cols[j]->fmap.size();
-    }
-    return BDF_OK;
-}
-
-static int fleet_chunk_info(bdf_ctx* c, const bdf_col* col, int64_t chunk, int64_t* len, int64_t* null_count, int32_t* has_validity);
-
-static int fleet_avg_dev(bdf_ctx* c, const bdf_col* col, double* out, int32_t* is_some) {
-    Fleet* f = c->fleet;
-    if (!is_fleet_col(col)) return fail(BDF_INVALID, "a column of a one-GPU context was passed to a multi-GPU context");
-    std::vector<double> v(f->kids.size(), 0.0);
-    std::vector<int32_t> some(f->kids.size(), 0);
-    TRY(fleet_run(f, [&](int k) { return bdf_avg_dev(f->kids[k], col->fparts[k], &v[k], &some[k]); }));
-    *out = v[0]; *is_some = some[0];
-    // aggregate.rs:57-60: `mean + (m - mean) * len / count` is 0/0 when the first chunk has no valid slot, and NaN sticks
-    if (!col->fmap.empty()) {
-        int64_t len = 0, nulls = 0; int32_t hv = 0;
-        TRY(fleet_chunk_info(c, col, 0, &len, &nulls, &hv));
-        if (len - (hv ? nulls : 0) == 0) *out = std::numeric_limits<double>::quiet_NaN();
-    }
-    return BDF_OK;
-}
-
-// Fused operator + aggregate: every kid runs the one-GPU entry on its parts; the future yields the global records.
-static int fleet_with_future(bdf_ctx* c, int out_dtype, std::initializer_list<const bdf_col*> inputs, bool want_col, bdf_col** out, bdf_future** fut,
-                             const std::function<int(int, bdf_col**, bdf_future**)>& call) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    const bdf_col* first = *inputs.begin();
-    int64_t n = (int64_t)first->fmap.size();
-    for (const bdf_col* col : inputs) {
-        if (!is_fleet_col(col)) return fail(BDF_INVALID, "a column of a one-GPU context was passed to a multi-GPU context");
-        n = std::min<int64_t>(n, (int64_t)col->fmap.size());
-    }
-    for (const bdf_col* col : inputs) {
-        for (int64_t i = 0; i < n; i++)
-            if (col->flens[i] != first->flens[i]) return fail(BDF_LENGTH_MISMATCH, "Cannot perform math operation on arrays of different length");
-        if (!fleet_same_map(first, col, n) || col->fmap.size() != first->fmap.size())
-            return fail(BDF_INVALID, "the columns are sharded differently over the GPUs (upload them in one bdf_upload_many call)");
-    }
-    bdf_col* o = want_col ? fleet_col_like(first, out_dtype, nk, n) : nullptr;
-    bdf_future* fu = fleet_future_new(nk);
-    if ((want_col && !o) || !fu) { fleet_col_free(f, o); delete fu; return fail(BDF_OOM, "host allocation failed"); }
-    fu->n = 1;
-    int st = fleet_run(f, [&](int k) { return call(k, o ? &o->fparts[k] : nullptr, &fu->fparts[k]); });
-    if (st != BDF_OK) {
-        const std::string keep = g_err;
-        fleet_future_wait(c, fu, nullptr);
-        fleet_col_free(f, o);
-        g_err = keep;
-        return st;
-    }
-    if (out) *out = o;
-    *fut = fu;
-    return BDF_OK;
-}
-
-// Host in / host out over every GPU: shard the views, run the one-GPU drop-in entry per kid (its own PCIe link), fold the metadata.
-static int fleet_binary_host(bdf_ctx* c, int op, int dtype, int64_t n_left, const bdf_view* left, int64_t n_right, const bdf_view* right, bdf_out* out) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    TRY(check_dtype(dtype));
-    if (n_left < 0 || n_right < 0 || (n_left && !left) || (n_right && !right)) return fail(BDF_INVALID, "bad arguments");
-    const int64_t n = std::min(n_left, n_right);
-    std::vector<int64_t> lens((size_t)n);
-    for (int64_t i = 0; i < n; i++) {
-        if (left[i].len != right[i].len) return fail(BDF_LENGTH_MISMATCH, "Cannot perform math operation on arrays of different length");
-        if (left[i].len < 0 || left[i].offset < 0 || right[i].offset < 0) return fail(BDF_INVALID, "bad view %lld", (long long)i);
-        lens[i] = left[i].len;
-    }
-    const auto map = fleet_plan(lens, nk);
-    std::vector<std::vector<bdf_view>> lv((size_t)nk), rv((size_t)nk);
-    std::vector<std::vector<bdf_out>> ov((size_t)nk);
-    for (int k = 0; k < nk; k++) { lv[k] = fleet_views(map, nk, k, left); rv[k] = fleet_views(map, nk, k, right); ov[k] = fleet_outs(map, k, dtype, out); }
-    TRY(fleet_run(f, [&](int k) {
-        bdf_view dv{}; bdf_out dummy{};
-        return bdf_binary(f->kids[k], op, dtype, (int64_t)lv[k].size(), lv[k].empty() ? &dv : lv[k].data(), (int64_t)rv[k].size(),
-                          rv[k].empty() ? &dv : rv[k].data(), ov[k].empty() ? &dummy : ov[k].data());
-    }));
-    fleet_merge_outs(map, ov, lens, out);
-    return BDF_OK;
-}
-
-static int fleet_map_host(bdf_ctx* c, bool is_cast, int op_or_to, int dtype, int64_t n, const bdf_view* in, bdf_out* out) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in)) return fail(BDF_INVALID, "bad arguments");
-    std::vector<int64_t> lens((size_t)n);
-    for (int64_t i = 0; i < n; i++) {
-        if (in[i].len < 0 || in[i].offset < 0) return fail(BDF_INVALID, "bad view %lld", (long long)i);
-        lens[i] = in[i].len;
-    }
-    const auto map = fleet_plan(lens, nk);
-    const int out_dtype = is_cast ? op_or_to : dtype;
-    std::vector<std::vector<bdf_view>> iv((size_t)nk);
-    std::vector<std::vector<bdf_out>> ov((size_t)nk);
-    for (int k = 0; k < nk; k++) { iv[k] = fleet_views(map, nk, k, in); ov[k] = fleet_outs(map, k, out_dtype, out); }
-    TRY(fleet_run(f, [&](int k) {
-        bdf_view dv{}; bdf_out dummy{};
-        const bdf_view* vp = iv[k].empty() ? &dv : iv[k].data();
-        bdf_out* op_ = ov[k].empty() ? &dummy : ov[k].data();
-        return is_cast ? bdf_cast(f->kids[k], dtype, op_or_to, (int64_t)iv[k].size(), vp, op_) : bdf_unary(f->kids[k], op_or_to, dtype, (int64_t)iv[k].size(), vp, op_);
-    }));
-    fleet_merge_outs(map, ov, lens, out);
-    return BDF_OK;
-}
-
-// Aggregates of a host column: upload the pieces (every GPU its own), reduce, combine; metadata rules over the caller's chunks.
-static int fleet_aggregate_host(bdf_ctx* c, int kind /* 0 one op, 1 all four, 2 avg */, int op, int dtype, int64_t n, const bdf_view* in, void* out_scalar,
-                                int32_t* is_some, bdf_agg4* all, double* avg) {
-    TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in)) return fail(BDF_INVALID, "bad arguments");
-    bdf_col* col = nullptr;
-    const int32_t dt = dtype;
-    const bdf_view* ptr = in;
-    TRY(fleet_upload_many(c, 1, &dt, &n, &ptr, BDF_ASYNC, &col));
-    int st;
-    if (kind == 0) st = fleet_aggregate_dev(c, op, col, out_scalar, is_some);
-    else if (kind == 1) { const bdf_col* cc = col; st = fleet_aggregate_all_blocking(c, 1, &cc, all); }
-    else st = fleet_avg_dev(c, col, avg, is_some);
-    const std::string keep = g_err;
-    Fleet* f = c->fleet;
-    fleet_run(f, [&](int k) { return bdf_col_wait(f->kids[k], col->fparts[k]); });   // host inputs must not be touched after return
-    fleet_col_free(f, col);
-    g_err = keep;
-    return st;
-}
-
-static int fleet_generate(bdf_ctx* c, int dtype, int kind, double lo, double hi, uint64_t seed, uint64_t col_id, int64_t n_chunks,
-                          const int64_t* chunk_lens, int64_t row0, uint32_t null_mod, bdf_col** out) {
-    Fleet* f = c->fleet;
-    const int nk = (int)f->kids.size();
-    std::vector<int64_t> lens((size_t)n_chunks);
-    for (int64_t i = 0; i < n_chunks; i++) { if (chunk_lens[i] < 0) return fail(BDF_INVALID, "negative chunk length"); lens[i] = chunk_lens[i]; }
-    bdf_col* col = fleet_col_new(dtype, nk);
-    if (!col) return fail(BDF_OOM, "host allocation failed");
-    col->fmap = fleet_plan(lens, nk);
-    col->flens = lens;
-    for (int64_t v : lens) col->total_len += v;
-    // a kid's pieces cover one contiguous range of global rows: generate them as one column starting at that row
-    std::vector<std::vector<int64_t>> klens((size_t)nk);
-    std::vector<int64_t> krow0((size_t)nk, -1);
-    int64_t start = 0;
-    for (int64_t i = 0; i < n_chunks; i++) {
-        for (const auto& pc : col->fmap[i]) {
-            if ((int64_t)klens[pc.kid].size() <= pc.local) klens[pc.kid].resize((size_t)pc.local + 1, 0);
-            klens[pc.kid][pc.local] = pc.rows;
-            if (krow0[pc.kid] < 0 && pc.rows > 0) krow0[pc.kid] = start + pc.row0;
-        }
-        start += lens[i];
-    }
-    int st = fleet_run(f, [&](int k) {
-        const int64_t dummy = 0;
-        return bdf_generate(f->kids[k], dtype, kind, lo, hi, seed, col_id, (int64_t)klens[k].size(), klens[k].empty() ? &dummy : klens[k].data(),
-                            row0 + std::max<int64_t>(krow0[k], 0), null_mod, &col->fparts[k]);
-    });
-    if (st != BDF_OK) { const std::string keep = g_err; fleet_col_free(f, col); g_err = keep; return st; }
-    *out = col;
-    return BDF_OK;
-}
-
-static int fleet_chunk_info(bdf_ctx* c, const bdf_col* col, int64_t chunk, int64_t* len, int64_t* null_count, int32_t* has_validity) {
-    Fleet* f = c->fleet;
-    if (!is_fleet_col(col) || chunk < 0 || chunk >= (int64_t)col->fmap.size()) return fail(BDF_INVALID, "bad chunk index");
-    if (len) *len = col->flens[chunk];
-    if (!null_count && !has_validity) return BDF_OK;
-    int64_t nulls = 0; int32_t hv = 0;
-    for (const auto& pc : col->fmap[chunk]) {   // a handful of pieces: the calling thread asks the kids in turn
-        int64_t l = 0, nc = 0; int32_t h = 0;
-        TRY(bdf_col_chunk_info(f->kids[pc.kid], col->fparts[pc.kid], pc.local, &l, null_count ? &nc : nullptr, &h));
-        nulls += nc; hv |= h;
-    }
-    if (null_count) *null_count = nulls;
-    if (has_validity) *has_validity = hv;
-    return BDF_OK;
-}
-
-static void fleet_destroy(bdf_ctx* c) {
-    Fleet* f = c->fleet;
-    for (auto& w : f->workers) {
-        { std::lock_guard<std::mutex> g(w->m); w->stop = true; }
-        w->cv.notify_all();
-        if (w->th.joinable()) w->th.join();
-    }
-    for (bdf_ctx* k : f->kids) bdf_destroy(k);
-    delete f;
-    delete c;
-}
-
-// ---------------------------------------------------------------------------------------------------
 // C ABI
+//
+// Every entry has one shape: the checks that need no device (context, pointers, counts, dtype codes, host views, the owner of
+// every column), then the dispatch of a multi-GPU context to fleet.cu, then ENTER and the one-GPU implementation.
+
+// sum/min/max/count: a known op, and min/max only where T::Native: Ord.
+static int check_agg_op(int op, int dtype) {
+    if (op < 0 || op >= BDF_NAGG) return fail(BDF_INVALID, "invalid aggregate op %d", op);
+    if ((op == BDF_MIN || op == BDF_MAX) && dtype_is_float(dtype)) return fail(BDF_UNSUPPORTED, "min/max need T::Native: Ord (integers only)");
+    return BDF_OK;
+}
+
+// Host in / host out on one GPU: upload the inputs, run fn on the device columns (a result column fn leaves in *o is downloaded
+// into out), release everything.
+static int host_call(bdf_ctx* c, const std::vector<UploadSpec>& specs, bdf_out* out, const std::function<int(bdf_col* const*, bdf_col**)>& fn) {
+    std::vector<bdf_col*> cols;
+    TRY(upload_many(c, specs, true, cols));
+    bdf_col* o = nullptr;
+    int st = fn(cols.data(), &o);
+    if (st == BDF_OK && o) st = download(c, o, out);
+    cudaStreamSynchronize(c->s_h2d);  // host inputs must not be touched after return
+    col_release(c, o);
+    for (bdf_col* col : cols) col_release(c, col);
+    return st;
+}
+
+namespace bdf { int ctx_attach_comm(bdf_ctx* c, Comm* cm) { c->comm = cm; c->collective = true; c->collectives = 0; return BDF_OK; } }
 
 #define ENTER(ctx)                                                   \
     if (!(ctx)) return fail(BDF_INVALID, "null context");           \
@@ -2501,8 +1803,8 @@ int bdf_abi_version(void) { return BDF_ABI_VERSION; }
 const char* bdf_last_error(void) { return g_err.c_str(); }
 
 void bdf_destroy(bdf_ctx* c) {
-    if (c && c->fleet) { fleet_destroy(c); return; }
     if (!c) return;
+    if (c->fleet) { fleet_destroy(c); return; }
     cudaSetDevice(c->device);
     if (c->s_compute) cudaStreamSynchronize(c->s_compute);
     if (c->s_h2d) cudaStreamSynchronize(c->s_h2d);
@@ -2598,65 +1900,8 @@ int bdf_init(int device, bdf_ctx** out) {
     return BDF_OK;
 }
 
-namespace bdf { int ctx_attach_comm(bdf_ctx* c, Comm* cm) { c->comm = cm; c->collective = true; c->collectives = 0; return BDF_OK; } }
-
-int bdf_init_multi(int n_gpus, const int* devices, bdf_ctx** out) {
-    if (!out) return fail(BDF_INVALID, "null out pointer");
-    *out = nullptr;
-    int n_dev = 0;
-    cudaError_t e = cudaGetDeviceCount(&n_dev);
-    if (e != cudaSuccess || n_dev == 0) {
-        cudaGetLastError();
-        return fail(BDF_CUDA, "no usable CUDA device (%s); this library has no CPU fallback", e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
-    }
-    if (n_gpus == 0) n_gpus = n_dev;
-    if (n_gpus < 1 || n_gpus > n_dev) return fail(BDF_INVALID, "%d GPUs requested, %d visible", n_gpus, n_dev);
-    std::vector<int> devs((size_t)n_gpus);
-    for (int i = 0; i < n_gpus; i++) {
-        devs[i] = devices ? devices[i] : i;
-        if (devs[i] < 0 || devs[i] >= n_dev) return fail(BDF_INVALID, "device %d out of range (0..%d)", devs[i], n_dev - 1);
-        for (int j = 0; j < i; j++) if (devs[j] == devs[i]) return fail(BDF_INVALID, "device %d listed twice", devs[i]);
-    }
-    bdf_ctx* c = new (std::nothrow) bdf_ctx();
-    Fleet* f = new (std::nothrow) Fleet();
-    if (!c || !f) { delete c; delete f; return fail(BDF_OOM, "host allocation failed"); }
-    c->fleet = f;
-    c->device = devs[0];
-    int st = BDF_OK;
-    for (int i = 0; i < n_gpus && st == BDF_OK; i++) {
-        bdf_ctx* kid = nullptr;
-        st = bdf_init(devs[i], &kid);
-        if (st == BDF_OK) f->kids.push_back(kid);
-    }
-    if (st == BDF_OK && n_gpus > 1) {   // ncclCommInitAll: one communicator, one rank per GPU, all in this process
-        std::vector<Comm*> comms((size_t)n_gpus, nullptr);
-        std::string err;
-        if (comm_create_all(n_gpus, devs.data(), comms.data(), &err) != 0) st = fail(BDF_NCCL, "%s", err.c_str());
-        else {
-            for (int i = 0; i < n_gpus; i++) ctx_attach_comm(f->kids[i], comms[i]);
-            const char* mode = getenv("BDF_COMBINE");
-            if (!(mode && strcmp(mode, "nccl") == 0)) {
-                std::string perr;
-                if (comm_enable_p2p_all(n_gpus, comms.data(), &perr) == 0) for (Comm* cm : comms) comm_set_p2p(cm, true);
-                else if (mode && strcmp(mode, "p2p") == 0) st = fail(BDF_NCCL, "BDF_COMBINE=p2p: %s", perr.c_str());
-            }
-        }
-    }
-    if (st == BDF_OK)
-        for (int i = 0; i < n_gpus; i++) {
-            f->workers.emplace_back(new Fleet::Worker());
-            Fleet::Worker* w = f->workers.back().get();
-            w->th = std::thread(fleet_worker_main, w, devs[i]);
-        }
-    if (st != BDF_OK) { const std::string keep = g_err; fleet_destroy(c); g_err = keep; return st; }
-    *out = c;
-    return BDF_OK;
-}
-
-int bdf_fleet_size(bdf_ctx* c) { return c ? (c->fleet ? (int)c->fleet->kids.size() : 1) : 0; }
-
 int bdf_synchronize(bdf_ctx* c) {
-    if (c && c->fleet) { Fleet* f = c->fleet; return fleet_run(f, [f](int k) { return bdf_synchronize(f->kids[k]); }); }
+    if (c && c->fleet) return fleet_each_gpu(c, bdf_synchronize);
     ENTER(c);
     CK(cudaStreamSynchronize(c->s_h2d));
     CK(cudaStreamSynchronize(c->s_compute));
@@ -2666,13 +1911,7 @@ int bdf_synchronize(bdf_ctx* c) {
 }
 
 int bdf_device_info(bdf_ctx* c, int32_t* sm_count, int32_t* cc_major, int32_t* cc_minor, int64_t* hbm_bytes) {
-    if (c && c->fleet) {   // the first GPU's shape, the HBM of all of them
-        int64_t total = 0, one = 0;
-        for (bdf_ctx* k : c->fleet->kids) { TRY(bdf_device_info(k, sm_count, cc_major, cc_minor, &one)); total += one; }
-        TRY(bdf_device_info(c->fleet->kids[0], sm_count, cc_major, cc_minor, &one));
-        if (hbm_bytes) *hbm_bytes = total;
-        return BDF_OK;
-    }
+    if (c && c->fleet) return fleet_device_info(c, sm_count, cc_major, cc_minor, hbm_bytes);
     if (!c) return fail(BDF_INVALID, "null context");
     if (sm_count) *sm_count = c->sm_count;
     if (cc_major) *cc_major = c->cc_major;
@@ -2682,26 +1921,26 @@ int bdf_device_info(bdf_ctx* c, int32_t* sm_count, int32_t* cc_major, int32_t* c
 }
 
 int bdf_host_alloc(bdf_ctx* c, size_t bytes, void** out) {
-    if (c && c->fleet) return bdf_host_alloc(c->fleet->kids[0], bytes, out);   // pinned memory is usable from every GPU (unified addressing)
+    if (c && c->fleet) return bdf_host_alloc(fleet_first_gpu(c), bytes, out);   // pinned memory is usable from every GPU (unified addressing)
     ENTER(c);
     if (!out) return fail(BDF_INVALID, "null out pointer");
     CK(cudaHostAlloc(out, bytes ? bytes : 1, cudaHostAllocDefault));
     return BDF_OK;
 }
 int bdf_host_free(bdf_ctx* c, void* p) {
-    if (c && c->fleet) return bdf_host_free(c->fleet->kids[0], p);
+    if (c && c->fleet) return bdf_host_free(fleet_first_gpu(c), p);
     ENTER(c);
     if (p) CK(cudaFreeHost(p));
     return BDF_OK;
 }
 int bdf_host_register(bdf_ctx* c, void* p, size_t bytes) {
-    if (c && c->fleet) return bdf_host_register(c->fleet->kids[0], p, bytes);
+    if (c && c->fleet) return bdf_host_register(fleet_first_gpu(c), p, bytes);
     ENTER(c);
     CK(cudaHostRegister(p, bytes, cudaHostRegisterDefault));
     return BDF_OK;
 }
 int bdf_host_unregister(bdf_ctx* c, void* p) {
-    if (c && c->fleet) return bdf_host_unregister(c->fleet->kids[0], p);
+    if (c && c->fleet) return bdf_host_unregister(fleet_first_gpu(c), p);
     ENTER(c);
     CK(cudaHostUnregister(p));
     return BDF_OK;
@@ -2743,7 +1982,7 @@ int bdf_comm_attach(bdf_ctx* c, const uint8_t* id, int rank, int world) {
 }
 
 int bdf_comm_set_combine(bdf_ctx* c, int mode) {
-    if (c && c->fleet) { for (bdf_ctx* k : c->fleet->kids) TRY(bdf_comm_set_combine(k, mode)); return BDF_OK; }
+    if (c && c->fleet) return fleet_each_gpu(c, [mode](bdf_ctx* k) { return bdf_comm_set_combine(k, mode); });
     ENTER(c);
     if (mode != 0 && mode != 1) return fail(BDF_INVALID, "combine mode is 0 (NCCL) or 1 (peer memory)");
     if (!c->comm) return mode == 0 ? BDF_OK : fail(BDF_UNSUPPORTED, "the context is not a rank of a communicator");
@@ -2754,7 +1993,7 @@ int bdf_comm_set_combine(bdf_ctx* c, int mode) {
 }
 
 int bdf_comm_get_combine(bdf_ctx* c) {
-    if (c && c->fleet) return bdf_comm_get_combine(c->fleet->kids[0]);
+    if (c && c->fleet) return bdf_comm_get_combine(fleet_first_gpu(c));
     return c && c->comm && comm_uses_p2p(c->comm) ? 1 : 0;
 }
 
@@ -2770,11 +2009,7 @@ int bdf_comm_detach(bdf_ctx* c) {
 }
 
 int bdf_comm_info(bdf_ctx* c, int32_t* rank, int32_t* world, int32_t* nccl_version, int64_t* collectives) {
-    if (c && c->fleet) {
-        TRY(bdf_comm_info(c->fleet->kids[0], rank, world, nccl_version, collectives));
-        if (rank) *rank = 0;
-        return BDF_OK;
-    }
+    if (c && c->fleet) return fleet_comm_info(c, rank, world, nccl_version, collectives);
     if (!c) return fail(BDF_INVALID, "null context");
     if (rank) *rank = c->comm ? comm_rank(c->comm) : 0;
     if (world) *world = c->comm ? comm_world(c->comm) : 1;
@@ -2816,16 +2051,20 @@ int bdf_comm_barrier(bdf_ctx* c) {
 }
 
 int bdf_aggregate_all_many_dev_async(bdf_ctx* c, int32_t n_cols, const bdf_col* const* cols, bdf_future** fut) {
-    if (c && c->fleet) { if (!cols || !fut) return fail(BDF_INVALID, "null argument"); return fleet_aggregate_many(c, n_cols, cols, fut); }
-    ENTER(c);
     if (!cols || !fut) return fail(BDF_INVALID, "null argument");
+    if (n_cols < 1 || n_cols > kCommMaxCols) return fail(BDF_INVALID, "an aggregate call takes 1..%d columns", kCommMaxCols);
+    TRY(check_cols(c, n_cols, cols));
+    if (c->fleet) return fleet_aggregate_many(c, n_cols, cols, fut);
+    ENTER(c);
     return aggregate_many_dev_async(c, n_cols, const_cast<bdf_col* const*>(cols), false, fut);
 }
 
 int bdf_aggregate_all_many_dev(bdf_ctx* c, int32_t n_cols, const bdf_col* const* cols, bdf_agg4* out) {
-    if (c && c->fleet) { if (!cols || !out) return fail(BDF_INVALID, "null argument"); return fleet_aggregate_all_blocking(c, n_cols, cols, out); }
-    ENTER(c);
     if (!cols || !out) return fail(BDF_INVALID, "null argument");
+    if (n_cols < 1 || n_cols > kCommMaxCols) return fail(BDF_INVALID, "an aggregate call takes 1..%d columns", kCommMaxCols);
+    TRY(check_cols(c, n_cols, cols));
+    if (c->fleet) return fleet_aggregate_all_blocking(c, n_cols, cols, out);
+    ENTER(c);
     bdf_future* f = nullptr;
     TRY(aggregate_many_dev_async(c, n_cols, const_cast<bdf_col* const*>(cols), true, &f));
     return future_wait(c, f, out);
@@ -2836,39 +2075,21 @@ int bdf_future_count(const bdf_future* fut) { return fut ? fut->n : 0; }
 // ---- device-resident API -----------------------------------------------------------------------
 
 int bdf_upload(bdf_ctx* c, int dtype, int64_t n_chunks, const bdf_view* in, int flags, bdf_col** out) {
-    if (c && c->fleet) {
-        if (dtype != kBool) TRY(check_dtype(dtype));
-        if (!out || n_chunks < 0 || (n_chunks && !in)) return fail(BDF_INVALID, "bad arguments");
-        const int32_t dt = dtype;
-        return fleet_upload_many(c, 1, &dt, &n_chunks, &in, flags, out);
-    }
-    ENTER(c);
-    if (dtype != kBool) TRY(check_dtype(dtype));
-    if (!out || n_chunks < 0 || (n_chunks && !in)) return fail(BDF_INVALID, "bad arguments");
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n_chunks, in}}, (flags & BDF_ASYNC) != 0, cols));
-    *out = cols[0];
-    return BDF_OK;
+    const int32_t dt = dtype;
+    return bdf_upload_many(c, 1, &dt, &n_chunks, &in, flags, out);
 }
 
 int bdf_upload_many(bdf_ctx* c, int64_t n_cols, const int32_t* dtypes, const int64_t* n_chunks, const bdf_view* const* in,
                     int flags, bdf_col** out) {
-    if (c && c->fleet) {
-        if (n_cols < 0 || (n_cols && (!dtypes || !n_chunks || !in || !out))) return fail(BDF_INVALID, "bad arguments");
-        for (int64_t k = 0; k < n_cols; k++) {
-            if (dtypes[k] != kBool) TRY(check_dtype(dtypes[k]));
-            if (n_chunks[k] < 0 || (n_chunks[k] && !in[k])) return fail(BDF_INVALID, "bad arguments for column %lld", (long long)k);
-        }
-        return fleet_upload_many(c, n_cols, dtypes, n_chunks, in, flags, out);
-    }
-    ENTER(c);
     if (n_cols < 0 || (n_cols && (!dtypes || !n_chunks || !in || !out))) return fail(BDF_INVALID, "bad arguments");
-    std::vector<UploadSpec> specs;
     for (int64_t k = 0; k < n_cols; k++) {
         if (dtypes[k] != kBool) TRY(check_dtype(dtypes[k]));
-        if (n_chunks[k] < 0 || (n_chunks[k] && !in[k])) return fail(BDF_INVALID, "bad arguments for column %lld", (long long)k);
-        specs.push_back(UploadSpec{dtypes[k], n_chunks[k], in[k]});
+        TRY(check_views(n_chunks[k], in[k]));
     }
+    if (c && c->fleet) return fleet_upload_many(c, n_cols, dtypes, n_chunks, in, flags, out);
+    ENTER(c);
+    std::vector<UploadSpec> specs;
+    for (int64_t k = 0; k < n_cols; k++) specs.push_back(UploadSpec{dtypes[k], n_chunks[k], in[k]});
     std::vector<bdf_col*> cols;
     TRY(upload_many(c, specs, (flags & BDF_ASYNC) != 0, cols));
     for (int64_t k = 0; k < n_cols; k++) out[k] = cols[k];
@@ -2876,31 +2097,26 @@ int bdf_upload_many(bdf_ctx* c, int64_t n_cols, const int32_t* dtypes, const int
 }
 
 int bdf_col_wait(bdf_ctx* c, const bdf_col* col) {
-    if (c && c->fleet) { if (!is_fleet_col(col)) return fail(BDF_INVALID, "null column"); Fleet* f = c->fleet; return fleet_run(f, [f, col](int k) { return bdf_col_wait(f->kids[k], col->fparts[k]); }); }
+    TRY(check_cols(c, {col}));
+    if (c->fleet) return fleet_col_wait(c, col);
     ENTER(c);
-    if (!col) return fail(BDF_INVALID, "null column");
     for (auto& g : col->groups) CK(cudaEventSynchronize(g.ev));
     return BDF_OK;
 }
 
 int bdf_col_describe(const bdf_col* col, int32_t* dtype, int64_t* n_chunks, int64_t* total_len) {
-    if (is_fleet_col(col)) {
-        if (dtype) *dtype = col->dtype;
-        if (n_chunks) *n_chunks = (int64_t)col->fmap.size();
-        if (total_len) *total_len = col->total_len;
-        return BDF_OK;
-    }
     if (!col) return fail(BDF_INVALID, "null column");
     if (dtype) *dtype = col->dtype;
-    if (n_chunks) *n_chunks = (int64_t)col->chunks.size();
+    if (n_chunks) *n_chunks = col_chunk_count(col);
     if (total_len) *total_len = col->total_len;
     return BDF_OK;
 }
 
 int bdf_col_chunk_info(bdf_ctx* c, const bdf_col* col, int64_t chunk, int64_t* len, int64_t* null_count, int32_t* has_validity) {
-    if (c && c->fleet) return fleet_chunk_info(c, col, chunk, len, null_count, has_validity);
+    TRY(check_cols(c, {col}));
+    if (chunk < 0 || chunk >= col_chunk_count(col)) return fail(BDF_INVALID, "bad chunk index");
+    if (c->fleet) return fleet_chunk_info(c, col, chunk, len, null_count, has_validity);
     ENTER(c);
-    if (!col || chunk < 0 || chunk >= (int64_t)col->chunks.size()) return fail(BDF_INVALID, "bad chunk index");
     if (len) *len = col->chunks[chunk].len;
     if (has_validity) *has_validity = col->chunks[chunk].validity != nullptr;
     if (null_count) {
@@ -2911,131 +2127,100 @@ int bdf_col_chunk_info(bdf_ctx* c, const bdf_col* col, int64_t chunk, int64_t* l
 }
 
 int bdf_binary_dev(bdf_ctx* c, int op, const bdf_col* l, const bdf_col* r, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!l || !r || !out) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        return fleet_map(c, l->dtype, {l, r}, out, [=](int k, bdf_col** o) { return bdf_binary_dev(f->kids[k], op, l->fparts[k], r->fparts[k], o); });
-    }
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {l, r}));
+    if (c->fleet) return fleet_binary_dev(c, op, l, r, out, nullptr);
     ENTER(c);
-    if (!l || !r || !out) return fail(BDF_INVALID, "null argument");
     return binary_dev(c, op, l, r, out);
 }
 
 int bdf_unary_dev(bdf_ctx* c, int op, const bdf_col* in, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!in || !out) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        return fleet_map(c, in->dtype, {in}, out, [=](int k, bdf_col** o) { return bdf_unary_dev(f->kids[k], op, in->fparts[k], o); });
-    }
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {in}));
+    if (c->fleet) return fleet_map_dev(c, false, op, in, out);
     ENTER(c);
-    if (!in || !out) return fail(BDF_INVALID, "null argument");
     return map_dev(c, false, op, in, out);
 }
 
 int bdf_cast_dev(bdf_ctx* c, int to, const bdf_col* in, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!in || !out) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        return fleet_map(c, to, {in}, out, [=](int k, bdf_col** o) { return bdf_cast_dev(f->kids[k], to, in->fparts[k], o); });
-    }
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {in}));
+    TRY(check_dtype(to));
+    if (c->fleet) return fleet_map_dev(c, true, to, in, out);
     ENTER(c);
-    if (!in || !out) return fail(BDF_INVALID, "null argument");
     return map_dev(c, true, to, in, out);
 }
 
 int bdf_aggregate_dev(bdf_ctx* c, int op, const bdf_col* in, void* out_scalar, int32_t* is_some) {
-    if (c && c->fleet) { if (!in || !out_scalar || !is_some) return fail(BDF_INVALID, "null argument"); return fleet_aggregate_dev(c, op, in, out_scalar, is_some); }
+    if (!out_scalar || !is_some) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {in}));
+    TRY(check_agg_op(op, in->dtype));
+    if (c->fleet) return fleet_aggregate_dev(c, op, in, out_scalar, is_some);
     ENTER(c);
-    if (!in || !out_scalar || !is_some) return fail(BDF_INVALID, "null argument");
     return aggregate_dev(c, op, const_cast<bdf_col*>(in), out_scalar, is_some);
 }
 
-int bdf_aggregate_all_dev(bdf_ctx* c, const bdf_col* in, bdf_agg4* out) {
-    if (c && c->fleet) { if (!in || !out) return fail(BDF_INVALID, "null argument"); return fleet_aggregate_all_blocking(c, 1, &in, out); }
-    ENTER(c);
-    if (!in || !out) return fail(BDF_INVALID, "null argument");
-    return aggregate_all_dev(c, const_cast<bdf_col*>(in), true, out);
-}
+int bdf_aggregate_all_dev(bdf_ctx* c, const bdf_col* in, bdf_agg4* out) { return bdf_aggregate_all_many_dev(c, 1, &in, out); }
 
 int bdf_avg_dev(bdf_ctx* c, const bdf_col* in, double* out, int32_t* is_some) {
-    if (c && c->fleet) { if (!in || !out || !is_some) return fail(BDF_INVALID, "null argument"); return fleet_avg_dev(c, in, out, is_some); }
+    if (!out || !is_some) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {in}));
+    if (c->fleet) return fleet_avg_dev(c, in, out, is_some);
     ENTER(c);
-    if (!in || !out || !is_some) return fail(BDF_INVALID, "null argument");
     return avg_dev(c, const_cast<bdf_col*>(in), out, is_some);
 }
 
 int bdf_binary_agg_dev_async(bdf_ctx* c, int op, const bdf_col* l, const bdf_col* r, bdf_col** out, bdf_future** fut) {
-    if (c && c->fleet) {
-        if (!l || !r || !out || !fut) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        return fleet_with_future(c, l->dtype, {l, r}, true, out, fut,
-                                 [=](int k, bdf_col** o, bdf_future** fu) { return bdf_binary_agg_dev_async(f->kids[k], op, l->fparts[k], r->fparts[k], o, fu); });
-    }
+    if (!out || !fut) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {l, r}));
+    if (c->fleet) return fleet_binary_dev(c, op, l, r, out, fut);
     ENTER(c);
-    if (!l || !r || !out || !fut) return fail(BDF_INVALID, "null argument");
     return binary_dev(c, op, l, r, out, fut);
 }
 
 int bdf_binary_agg_dev(bdf_ctx* c, int op, const bdf_col* l, const bdf_col* r, bdf_col** out, bdf_agg4* agg) {
-    if (c && c->fleet) {
-        if (!l || !r || !out || !agg) return fail(BDF_INVALID, "null argument");
-        bdf_future* fu = nullptr;
-        TRY(bdf_binary_agg_dev_async(c, op, l, r, out, &fu));
-        return fleet_future_wait(c, fu, agg);
-    }
-    ENTER(c);
-    if (!l || !r || !out || !agg) return fail(BDF_INVALID, "null argument");
+    if (!agg) return fail(BDF_INVALID, "null argument");
     bdf_future* f = nullptr;
-    TRY(binary_dev(c, op, l, r, out, &f));
-    return future_wait(c, f, agg);
+    TRY(bdf_binary_agg_dev_async(c, op, l, r, out, &f));
+    return bdf_future_wait(c, f, agg);
+}
+
+// The two expression entries (fut == nullptr: bdf_eval_expr_dev).
+static int expr_entry(bdf_ctx* c, int n_inputs, const bdf_col* const* inputs, int n_nodes, const bdf_expr_node* nodes, bdf_col** out,
+                      bdf_future** fut) {
+    if (!inputs || !nodes) return fail(BDF_INVALID, "null argument");
+    int in_dtypes[8] = {0};
+    const int n = std::max(0, std::min(n_inputs, 8));   // expr_prepare rejects any other count
+    TRY(check_cols(c, n, inputs));
+    for (int i = 0; i < n; i++) in_dtypes[i] = inputs[i]->dtype;
+    alignas(8) unsigned char prog[256];
+    bool has_div = false;
+    TRY(expr_prepare(n_inputs, in_dtypes, n_nodes, nodes, prog, &has_div));
+    if (c->fleet) return fleet_eval_expr(c, n_inputs, inputs, n_nodes, nodes, out, fut);
+    ENTER(c);
+    return expr_dev(c, n_inputs, inputs, prog, has_div, out, fut);
 }
 
 int bdf_eval_expr_agg_dev_async(bdf_ctx* c, int32_t n_inputs, const bdf_col* const* inputs, int32_t n_nodes, const bdf_expr_node* nodes,
                                 bdf_col** out, bdf_future** fut) {
-    if (c && c->fleet) {
-        if (!inputs || !nodes || !fut || n_inputs < 1 || n_inputs > 8) return fail(BDF_INVALID, "bad arguments");
-        for (int i = 0; i < n_inputs; i++) if (!is_fleet_col(inputs[i])) return fail(BDF_INVALID, "null input column");
-        for (int i = 1; i < n_inputs; i++)
-            if (inputs[i]->fmap.size() != inputs[0]->fmap.size() || !fleet_same_map(inputs[0], inputs[i], (int64_t)inputs[0]->fmap.size()))
-                return fail(BDF_INVALID, "the columns are sharded differently over the GPUs (upload them in one bdf_upload_many call)");
-        Fleet* f = c->fleet;
-        return fleet_with_future(c, BDF_F64, {inputs[0]}, out != nullptr, out, fut, [=](int k, bdf_col** o, bdf_future** fu) {
-            const bdf_col* parts[8];
-            for (int i = 0; i < n_inputs; i++) parts[i] = inputs[i]->fparts[k];
-            return bdf_eval_expr_agg_dev_async(f->kids[k], n_inputs, parts, n_nodes, nodes, o, fu);
-        });
-    }
-    ENTER(c);
-    if (!inputs || !nodes || !fut) return fail(BDF_INVALID, "null argument");
-    return expr_dev(c, n_inputs, inputs, n_nodes, nodes, out, fut);
+    if (!fut) return fail(BDF_INVALID, "null argument");
+    return expr_entry(c, n_inputs, inputs, n_nodes, nodes, out, fut);
 }
 
 int bdf_eval_expr_agg_dev(bdf_ctx* c, int32_t n_inputs, const bdf_col* const* inputs, int32_t n_nodes, const bdf_expr_node* nodes, bdf_col** out,
                           bdf_agg4* agg) {
-    if (c && c->fleet) {
-        if (!agg) return fail(BDF_INVALID, "null argument");
-        bdf_future* fu = nullptr;
-        TRY(bdf_eval_expr_agg_dev_async(c, n_inputs, inputs, n_nodes, nodes, out, &fu));
-        return fleet_future_wait(c, fu, agg);
-    }
-    ENTER(c);
-    if (!inputs || !nodes || !agg) return fail(BDF_INVALID, "null argument");
+    if (!agg) return fail(BDF_INVALID, "null argument");
     bdf_future* f = nullptr;
-    TRY(expr_dev(c, n_inputs, inputs, n_nodes, nodes, out, &f));
-    return future_wait(c, f, agg);
+    TRY(bdf_eval_expr_agg_dev_async(c, n_inputs, inputs, n_nodes, nodes, out, &f));
+    return bdf_future_wait(c, f, agg);
 }
 
-int bdf_aggregate_all_dev_async(bdf_ctx* c, const bdf_col* in, bdf_future** fut) {
-    if (c && c->fleet) { if (!in || !fut) return fail(BDF_INVALID, "null argument"); return fleet_aggregate_many(c, 1, &in, fut); }
-    ENTER(c);
-    if (!in || !fut) return fail(BDF_INVALID, "null argument");
-    return aggregate_all_dev_async(c, const_cast<bdf_col*>(in), fut);
-}
+int bdf_aggregate_all_dev_async(bdf_ctx* c, const bdf_col* in, bdf_future** fut) { return bdf_aggregate_all_many_dev_async(c, 1, &in, fut); }
 
 int bdf_future_wait(bdf_ctx* c, bdf_future* fut, bdf_agg4* out) {
-    if (c && c->fleet) { if (!fut) return fail(BDF_INVALID, "null future"); return fleet_future_wait(c, fut, out); }
-    ENTER(c);
     if (!fut) return fail(BDF_INVALID, "null future");
+    if (c && c->fleet) return fleet_future_wait(c, fut, out);
+    ENTER(c);
     return future_wait(c, fut, out);
 }
 
@@ -3055,101 +2240,80 @@ int bdf_expr_check(int32_t n_inputs, const int32_t* input_dtypes, int32_t n_node
 }
 
 int bdf_eval_expr_dev(bdf_ctx* c, int32_t n_inputs, const bdf_col* const* inputs, int32_t n_nodes, const bdf_expr_node* nodes, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!inputs || !nodes || !out || n_inputs < 1 || n_inputs > 8) return fail(BDF_INVALID, "bad arguments");
-        for (int i = 0; i < n_inputs; i++) if (!is_fleet_col(inputs[i])) return fail(BDF_INVALID, "null input column");
-        for (int i = 1; i < n_inputs; i++)
-            if (inputs[i]->fmap.size() != inputs[0]->fmap.size() || !fleet_same_map(inputs[0], inputs[i], (int64_t)inputs[0]->fmap.size()))
-                return fail(BDF_INVALID, "the columns are sharded differently over the GPUs (upload them in one bdf_upload_many call)");
-        Fleet* f = c->fleet;
-        return fleet_map(c, BDF_F64, {inputs[0]}, out, [=](int k, bdf_col** o) {
-            const bdf_col* parts[8];
-            for (int i = 0; i < n_inputs; i++) parts[i] = inputs[i]->fparts[k];
-            return bdf_eval_expr_dev(f->kids[k], n_inputs, parts, n_nodes, nodes, o);
-        });
-    }
-    ENTER(c);
-    if (!inputs || !nodes || !out) return fail(BDF_INVALID, "null argument");
-    return expr_dev(c, n_inputs, inputs, n_nodes, nodes, out);
+    if (!out) return fail(BDF_INVALID, "null argument");
+    return expr_entry(c, n_inputs, inputs, n_nodes, nodes, out, nullptr);
 }
 
 int bdf_sort_indices_dev(bdf_ctx* c, int32_t n_keys, const bdf_sort_key* keys, bdf_col** indices) {
+    if (!keys || !indices) return fail(BDF_INVALID, "null argument");
+    for (int32_t k = 0; k < n_keys; k++) TRY(check_cols(c, {keys[k].column}));
     if (c && c->fleet) return fail(BDF_UNSUPPORTED, "sort / take / filter move rows between chunks: use a one-GPU context (bdf_init) for them");
     ENTER(c);
-    if (!keys || !indices) return fail(BDF_INVALID, "null argument");
     return sort_indices_dev(c, n_keys, keys, indices);
 }
 
 int bdf_group_aggregate_dev(bdf_ctx* c, const bdf_col* key, int32_t n_values, const bdf_col* const* values, bdf_col** out_keys, bdf_group_out* out,
                             int64_t* n_groups) {
-    if (c && c->fleet) return fail(BDF_UNSUPPORTED, "group-by moves rows between chunks: use a one-GPU context (bdf_init) for it");
+    if (!out_keys || (n_values && (!values || !out))) return fail(BDF_INVALID, "null argument");
+    if (n_values < 0 || n_values > 64) return fail(BDF_INVALID, "0..64 value columns");
+    TRY(check_cols(c, {key}));
+    TRY(check_cols(c, n_values, values));
+    if (c->fleet) return fail(BDF_UNSUPPORTED, "group-by moves rows between chunks: use a one-GPU context (bdf_init) for it");
     ENTER(c);
-    if (!key || !out_keys || (n_values && (!values || !out))) return fail(BDF_INVALID, "null argument");
     return group_aggregate_dev(c, key, n_values, values, out_keys, out, n_groups);
 }
 
 int bdf_take_dev(bdf_ctx* c, const bdf_col* values, const bdf_col* indices, bdf_col** out) {
-    if (c && c->fleet) return fail(BDF_UNSUPPORTED, "sort / take / filter move rows between chunks: use a one-GPU context (bdf_init) for them");
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {values, indices}));
+    if (c->fleet) return fail(BDF_UNSUPPORTED, "sort / take / filter move rows between chunks: use a one-GPU context (bdf_init) for them");
     ENTER(c);
-    if (!values || !indices || !out) return fail(BDF_INVALID, "null argument");
     return take_dev(c, values, indices, out);
 }
 
 int bdf_compare_dev(bdf_ctx* c, int op, const bdf_col* left, const bdf_col* right, double scalar, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!left || !out) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        if (right) return fleet_map(c, kBool, {left, right}, out, [=](int k, bdf_col** o) { return bdf_compare_dev(f->kids[k], op, left->fparts[k], right->fparts[k], scalar, o); });
-        return fleet_map(c, kBool, {left}, out, [=](int k, bdf_col** o) { return bdf_compare_dev(f->kids[k], op, left->fparts[k], nullptr, scalar, o); });
-    }
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {left}));
+    if (right) TRY(check_cols(c, {right}));
+    if (c->fleet) return fleet_compare_dev(c, op, left, right, scalar, out);
     ENTER(c);
-    if (!left || !out) return fail(BDF_INVALID, "null argument");
     return compare_dev(c, op, left, right, scalar, out);
 }
 
 int bdf_boolean_dev(bdf_ctx* c, int op, const bdf_col* a, const bdf_col* b, bdf_col** out) {
-    if (c && c->fleet) {
-        if (!a || !out) return fail(BDF_INVALID, "null argument");
-        Fleet* f = c->fleet;
-        if (b && op != BDF_NOT) return fleet_map(c, kBool, {a, b}, out, [=](int k, bdf_col** o) { return bdf_boolean_dev(f->kids[k], op, a->fparts[k], b->fparts[k], o); });
-        return fleet_map(c, kBool, {a}, out, [=](int k, bdf_col** o) { return bdf_boolean_dev(f->kids[k], op, a->fparts[k], nullptr, o); });
-    }
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {a}));
+    if (b) TRY(check_cols(c, {b}));
+    if (c->fleet) return fleet_boolean_dev(c, op, a, b, out);
     ENTER(c);
-    if (!a || !out) return fail(BDF_INVALID, "null argument");
     return boolean_dev(c, op, a, b, out);
 }
 
 int bdf_filter_dev(bdf_ctx* c, const bdf_col* values, const bdf_col* mask, bdf_col** out) {
-    if (c && c->fleet) return fail(BDF_UNSUPPORTED, "sort / take / filter move rows between chunks: use a one-GPU context (bdf_init) for them");
+    if (!out) return fail(BDF_INVALID, "null argument");
+    TRY(check_cols(c, {values, mask}));
+    if (c->fleet) return fail(BDF_UNSUPPORTED, "sort / take / filter move rows between chunks: use a one-GPU context (bdf_init) for them");
     ENTER(c);
-    if (!values || !mask || !out) return fail(BDF_INVALID, "null argument");
     return filter_dev(c, values, mask, out);
 }
 
-int bdf_download_begin(bdf_ctx* c, const bdf_col* col, bdf_out* out) {
-    if (c && c->fleet) { if (!is_fleet_col(col) || (!out && !col->fmap.empty())) return fail(BDF_INVALID, "null argument"); return fleet_download(c, col, out, 1); }
+// The three download entries (phase 0 both halves, 1 begin, 2 end).
+static int download_entry(bdf_ctx* c, const bdf_col* col, bdf_out* out, int phase) {
+    TRY(check_cols(c, {col}));
+    if (!out && col_chunk_count(col)) return fail(BDF_INVALID, "null argument");
+    if (c->fleet) return fleet_download(c, col, out, phase);
     ENTER(c);
-    if (!col || (!out && !col->chunks.empty())) return fail(BDF_INVALID, "null argument");
-    return download_enqueue(c, const_cast<bdf_col*>(col), out);
+    bdf_col* m = const_cast<bdf_col*>(col);
+    return phase == 1 ? download_enqueue(c, m, out) : phase == 2 ? download_finish(c, m, out) : download(c, m, out);
 }
 
-int bdf_download_end(bdf_ctx* c, const bdf_col* col, bdf_out* out) {
-    if (c && c->fleet) { if (!is_fleet_col(col) || (!out && !col->fmap.empty())) return fail(BDF_INVALID, "null argument"); return fleet_download(c, col, out, 2); }
-    ENTER(c);
-    if (!col || (!out && !col->chunks.empty())) return fail(BDF_INVALID, "null argument");
-    return download_finish(c, const_cast<bdf_col*>(col), out);
-}
-
-int bdf_download(bdf_ctx* c, const bdf_col* col, bdf_out* out) {
-    if (c && c->fleet) { if (!is_fleet_col(col) || (!out && !col->fmap.empty())) return fail(BDF_INVALID, "null argument"); return fleet_download(c, col, out, 0); }
-    ENTER(c);
-    if (!col || (!out && !col->chunks.empty())) return fail(BDF_INVALID, "null argument");
-    return download(c, const_cast<bdf_col*>(col), out);
-}
+int bdf_download_begin(bdf_ctx* c, const bdf_col* col, bdf_out* out) { return download_entry(c, col, out, 1); }
+int bdf_download_end(bdf_ctx* c, const bdf_col* col, bdf_out* out) { return download_entry(c, col, out, 2); }
+int bdf_download(bdf_ctx* c, const bdf_col* col, bdf_out* out) { return download_entry(c, col, out, 0); }
 
 void bdf_col_free(bdf_ctx* c, bdf_col* col) {
-    if (c && c->fleet) { fleet_col_free(c->fleet, col); return; }
     if (!c || !col) return;
+    if (c->fleet) { fleet_col_free(c, col); return; }
     std::lock_guard<std::mutex> lock(c->mu);
     cudaSetDevice(c->device);
     col_release(c, col);
@@ -3158,57 +2322,44 @@ void bdf_col_free(bdf_ctx* c, bdf_col* col) {
 // ---- host in / host out ------------------------------------------------------------------------
 
 int bdf_binary(bdf_ctx* c, int op, int dtype, int64_t n_left, const bdf_view* left, int64_t n_right, const bdf_view* right, bdf_out* out) {
-    if (c && c->fleet) { if (!out && std::min(n_left, n_right) > 0) return fail(BDF_INVALID, "bad arguments"); return fleet_binary_host(c, op, dtype, n_left, left, n_right, right, out); }
-    ENTER(c);
     TRY(check_dtype(dtype));
     if (n_left < 0 || n_right < 0 || (n_left && !left) || (n_right && !right)) return fail(BDF_INVALID, "bad arguments");
-    const int64_t n = std::min(n_left, n_right);
+    const int64_t n = std::min(n_left, n_right);   // zip()
+    if (n && !out) return fail(BDF_INVALID, "bad arguments");
+    TRY(check_views(n, left));
+    TRY(check_views(n, right));
     for (int64_t i = 0; i < n; i++)  // reject before moving a byte
         if (left[i].len != right[i].len) return fail(BDF_LENGTH_MISMATCH, "Cannot perform math operation on arrays of different length");
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n, left}, UploadSpec{dtype, n, right}}, true, cols));
-    bdf_col* o = nullptr;
-    int st = binary_dev(c, op, cols[0], cols[1], &o);
-    if (st == BDF_OK) st = download(c, o, out);
-    std::string keep = g_err;
-    cudaStreamSynchronize(c->s_h2d);  // host inputs must not be touched after return
-    col_release(c, o); col_release(c, cols[0]); col_release(c, cols[1]);
-    g_err = keep;
-    return st;
-}
-
-static int map_host(bdf_ctx* c, bool is_cast, int op_or_to, int dtype, int64_t n, const bdf_view* in, bdf_out* out) {
-    TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in)) return fail(BDF_INVALID, "bad arguments");
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n, in}}, true, cols));
-    bdf_col* o = nullptr;
-    int st = map_dev(c, is_cast, op_or_to, cols[0], &o);
-    if (st == BDF_OK) st = download(c, o, out);
-    std::string keep = g_err;
-    cudaStreamSynchronize(c->s_h2d);
-    col_release(c, o); col_release(c, cols[0]);
-    g_err = keep;
-    return st;
+    if (c && c->fleet) return fleet_binary_host(c, op, dtype, n, left, right, out);
+    ENTER(c);
+    return host_call(c, {UploadSpec{dtype, n, left}, UploadSpec{dtype, n, right}}, out,
+                     [&](bdf_col* const* in, bdf_col** o) { return binary_dev(c, op, in[0], in[1], o); });
 }
 
 int bdf_unary(bdf_ctx* c, int op, int dtype, int64_t n, const bdf_view* in, bdf_out* out) {
+    TRY(check_dtype(dtype));
+    TRY(check_views(n, in));
     if (c && c->fleet) return fleet_map_host(c, false, op, dtype, n, in, out);
     ENTER(c);
-    return map_host(c, false, op, dtype, n, in, out);
+    return host_call(c, {UploadSpec{dtype, n, in}}, out, [&](bdf_col* const* cols, bdf_col** o) { return map_dev(c, false, op, cols[0], o); });
 }
 
 int bdf_cast(bdf_ctx* c, int from, int to, int64_t n, const bdf_view* in, bdf_out* out) {
-    if (c && c->fleet) { TRY(check_dtype(to)); return fleet_map_host(c, true, to, from, n, in, out); }
+    TRY(check_dtype(from));
+    TRY(check_dtype(to));
+    TRY(check_views(n, in));
+    if (c && c->fleet) return fleet_map_host(c, true, to, from, n, in, out);
     ENTER(c);
-    return map_host(c, true, to, from, n, in, out);
+    return host_call(c, {UploadSpec{from, n, in}}, out, [&](bdf_col* const* cols, bdf_col** o) { return map_dev(c, true, to, cols[0], o); });
 }
 
 int bdf_aggregate(bdf_ctx* c, int op, int dtype, int64_t n, const bdf_view* in, void* out_scalar, int32_t* is_some) {
-    if (c && c->fleet) { if (!out_scalar || !is_some) return fail(BDF_INVALID, "bad arguments"); return fleet_aggregate_host(c, 0, op, dtype, n, in, out_scalar, is_some, nullptr, nullptr); }
-    ENTER(c);
     TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in) || !out_scalar || !is_some) return fail(BDF_INVALID, "bad arguments");
+    TRY(check_views(n, in));
+    if (!out_scalar || !is_some) return fail(BDF_INVALID, "bad arguments");
+    TRY(check_agg_op(op, dtype));
+    if (c && c->fleet) return fleet_aggregate_host(c, dtype, n, in, [&](const bdf_col* col) { return bdf_aggregate_dev(c, op, col, out_scalar, is_some); });
+    ENTER(c);
     if (op == BDF_COUNT) {  // metadata only when every null_count is known: no bytes move
         bool known = true;
         int64_t total = 0;
@@ -3218,66 +2369,39 @@ int bdf_aggregate(bdf_ctx* c, int op, int dtype, int64_t n, const bdf_view* in, 
         }
         if (known) { TRY(count_global(c, &total)); *(int64_t*)out_scalar = total; *is_some = 1; return BDF_OK; }
     }
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n, in}}, true, cols));
-    int st = aggregate_dev(c, op, cols[0], out_scalar, is_some);
-    std::string keep = g_err;
-    cudaStreamSynchronize(c->s_h2d);
-    col_release(c, cols[0]);
-    g_err = keep;
-    return st;
+    return host_call(c, {UploadSpec{dtype, n, in}}, nullptr,
+                     [&](bdf_col* const* cols, bdf_col**) { return aggregate_dev(c, op, cols[0], out_scalar, is_some); });
 }
 
 int bdf_aggregate_all(bdf_ctx* c, int dtype, int64_t n, const bdf_view* in, bdf_agg4* out) {
-    if (c && c->fleet) { if (!out) return fail(BDF_INVALID, "bad arguments"); return fleet_aggregate_host(c, 1, 0, dtype, n, in, nullptr, nullptr, out, nullptr); }
-    ENTER(c);
     TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in) || !out) return fail(BDF_INVALID, "bad arguments");
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n, in}}, true, cols));
-    int st = aggregate_all_dev(c, cols[0], true, out);
-    std::string keep = g_err;
-    cudaStreamSynchronize(c->s_h2d);
-    col_release(c, cols[0]);
-    g_err = keep;
-    return st;
+    TRY(check_views(n, in));
+    if (!out) return fail(BDF_INVALID, "bad arguments");
+    if (c && c->fleet) return fleet_aggregate_host(c, dtype, n, in, [&](const bdf_col* col) { return bdf_aggregate_all_dev(c, col, out); });
+    ENTER(c);
+    return host_call(c, {UploadSpec{dtype, n, in}}, nullptr, [&](bdf_col* const* cols, bdf_col**) { return aggregate_all_dev(c, cols[0], true, out); });
 }
 
 int bdf_avg(bdf_ctx* c, int dtype, int64_t n, const bdf_view* in, double* out, int32_t* is_some) {
-    if (c && c->fleet) { if (!out || !is_some) return fail(BDF_INVALID, "bad arguments"); return fleet_aggregate_host(c, 2, 0, dtype, n, in, nullptr, is_some, nullptr, out); }
-    ENTER(c);
     TRY(check_dtype(dtype));
-    if (n < 0 || (n && !in) || !out || !is_some) return fail(BDF_INVALID, "bad arguments");
-    std::vector<bdf_col*> cols;
-    TRY(upload_many(c, {UploadSpec{dtype, n, in}}, true, cols));
-    int st = avg_dev(c, cols[0], out, is_some);
-    std::string keep = g_err;
-    cudaStreamSynchronize(c->s_h2d);
-    col_release(c, cols[0]);
-    g_err = keep;
-    return st;
+    TRY(check_views(n, in));
+    if (!out || !is_some) return fail(BDF_INVALID, "bad arguments");
+    if (c && c->fleet) return fleet_aggregate_host(c, dtype, n, in, [&](const bdf_col* col) { return bdf_avg_dev(c, col, out, is_some); });
+    ENTER(c);
+    return host_call(c, {UploadSpec{dtype, n, in}}, nullptr, [&](bdf_col* const* cols, bdf_col**) { return avg_dev(c, cols[0], out, is_some); });
 }
 
 // ---- measurement support -------------------------------------------------------------------------
 
 int bdf_profile_enable(bdf_ctx* c, int on) {
-    if (c && c->fleet) { for (bdf_ctx* k : c->fleet->kids) TRY(bdf_profile_enable(k, on)); return BDF_OK; }
+    if (c && c->fleet) return fleet_each_gpu(c, [on](bdf_ctx* k) { return bdf_profile_enable(k, on); });
     ENTER(c);
     c->profiling = on != 0;
     return BDF_OK;
 }
 
 int bdf_profile_read(bdf_ctx* c, bdf_launch_record* buf, int64_t cap, int64_t* n) {
-    if (c && c->fleet) {   // the records of all GPUs, GPU by GPU
-        int64_t total = 0;
-        for (bdf_ctx* k : c->fleet->kids) {
-            int64_t got = 0;
-            TRY(bdf_profile_read(k, buf ? buf + total : nullptr, buf ? cap - total : 0, &got));
-            total += got;
-        }
-        if (n) *n = total;
-        return BDF_OK;
-    }
+    if (c && c->fleet) return fleet_profile_read(c, buf, cap, n);
     ENTER(c);
     CK(cudaStreamSynchronize(c->s_compute));
     int64_t k = 0;
@@ -3294,24 +2418,19 @@ int bdf_profile_read(bdf_ctx* c, bdf_launch_record* buf, int64_t cap, int64_t* n
 }
 
 int64_t bdf_launch_count(bdf_ctx* c) {
-    if (c && c->fleet) { int64_t t = 0; for (bdf_ctx* k : c->fleet->kids) t += bdf_launch_count(k); return t; }
+    if (c && c->fleet) return fleet_launch_count(c);
     return c ? c->launches : 0;
 }
 
 int bdf_timer_start(bdf_ctx* c) {
-    if (c && c->fleet) { for (bdf_ctx* k : c->fleet->kids) TRY(bdf_timer_start(k)); return BDF_OK; }
+    if (c && c->fleet) return fleet_each_gpu(c, bdf_timer_start);
     ENTER(c);
     CK(cudaEventRecord(c->ev_t0, c->s_compute));
     return BDF_OK;
 }
 
 int bdf_timer_stop(bdf_ctx* c, float* ms) {
-    if (c && c->fleet) {   // the slowest GPU
-        float worst = 0.f;
-        for (bdf_ctx* k : c->fleet->kids) { float one = 0.f; TRY(bdf_timer_stop(k, &one)); worst = std::max(worst, one); }
-        if (ms) *ms = worst;
-        return BDF_OK;
-    }
+    if (c && c->fleet) return fleet_timer_stop(c, ms);
     ENTER(c);
     CK(cudaEventRecord(c->ev_t1, c->s_compute));
     CK(cudaEventSynchronize(c->ev_t1));
@@ -3320,7 +2439,7 @@ int bdf_timer_stop(bdf_ctx* c, float* ms) {
 }
 
 int bdf_flush_l2(bdf_ctx* c, size_t bytes) {
-    if (c && c->fleet) { for (bdf_ctx* k : c->fleet->kids) TRY(bdf_flush_l2(k, bytes)); return BDF_OK; }
+    if (c && c->fleet) return fleet_each_gpu(c, [bytes](bdf_ctx* k) { return bdf_flush_l2(k, bytes); });
     ENTER(c);
     if (bytes > c->flush_bytes) {
         if (c->flush_buf) CK(cudaFree(c->flush_buf));
@@ -3334,19 +2453,14 @@ int bdf_flush_l2(bdf_ctx* c, size_t bytes) {
 
 int bdf_generate(bdf_ctx* c, int dtype, int kind, double lo, double hi, uint64_t seed, uint64_t col_id, int64_t n_chunks,
                  const int64_t* chunk_lens, int64_t row0, uint32_t null_mod, bdf_col** out) {
-    if (c && c->fleet) {
-        TRY(check_dtype(dtype));
-        if (!out || n_chunks < 0 || (n_chunks && !chunk_lens) || kind < 0 || kind > 3) return fail(BDF_INVALID, "bad arguments");
-        return fleet_generate(c, dtype, kind, lo, hi, seed, col_id, n_chunks, chunk_lens, row0, null_mod, out);
-    }
-    ENTER(c);
     TRY(check_dtype(dtype));
     if (!out || n_chunks < 0 || (n_chunks && !chunk_lens) || kind < 0 || kind > 3) return fail(BDF_INVALID, "bad arguments");
-    std::vector<ChunkPlan> plan((size_t)n_chunks);
-    for (int64_t i = 0; i < n_chunks; i++) {
+    for (int64_t i = 0; i < n_chunks; i++)
         if (chunk_lens[i] < 0) return fail(BDF_INVALID, "negative chunk length");
-        plan[i] = {chunk_lens[i], null_mod != 0};
-    }
+    if (c && c->fleet) return fleet_generate(c, dtype, kind, lo, hi, seed, col_id, n_chunks, chunk_lens, row0, null_mod, out);
+    ENTER(c);
+    std::vector<ChunkPlan> plan((size_t)n_chunks);
+    for (int64_t i = 0; i < n_chunks; i++) plan[i] = {chunk_lens[i], null_mod != 0};
     bdf_col* o = nullptr;
     const int tile = elems_per_tile(dtype);
     TRY(col_alloc(c, dtype, plan, nullptr, tile, &o));
